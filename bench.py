@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the GN-ODE rollout hot path (BASELINE.json metric: rollout node-steps/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 Workload (config.workload): BASELINE.json configs[3] as written -- epinions-scale rollout inference of 4096 trials
@@ -17,12 +17,21 @@ Prints ONE JSON line (rank 0). value = node-steps/s with every descriptor reside
 grid points left in HBM; e2e = the same job through ODEBlock.forward_trials with the descriptors in pinned host memory
 and the probabilities of the grid points the reference's test() consumes (get_sir_t_nodes_torch: rows int(i/deltaT),
 20 of 40) copied back to pinned host memory inside the timed region.
+
+--dump-outputs DIR writes what the last timed step of the device-resident measurement computed: the probabilities
+[T, rows, 3] (S, I, R at every grid point) of DUMP_ROWS (trial, node) rows drawn with a fixed seed from the whole job, as
+DIR/probs_sample.npy (float32), and their row ids trial * N + node as DIR/probs_sample_rows.npy (float64); under several
+ranks each rank writes its own share with the suffix _rank<r>. The rows are gathered on the device after each chunk of
+that step, one small index_select per chunk inside the timed window.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -45,6 +54,7 @@ R_STATE_NOTE = {
 JSON_OUT = sys.stdout
 UNIT = "node-steps/s"
 METRIC = "GN-ODE rollout node-steps/s (epinions)"
+DUMP_ROWS = 65536                      # x T x 3 float32 = 31.5 MB for T = 40
 
 
 def measured_peak():
@@ -328,7 +338,13 @@ def main():
     ap.add_argument("--ref-trials", type=int, default=2)
     ap.add_argument("--ref-points", type=int, default=20)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample of what the last timed step computed to DIR/*.npy (--mode rollout)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "rollout"):
+        ap.error("--dump-outputs needs --impl ours --mode rollout")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -356,8 +372,13 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     import gn_ode_sir_b200 as gn
-    from gn_ode_sir_b200 import _lib
-    gn.build_library()
+    from gn_ode_sir_b200 import _build, _lib
+    if "GNODE_B200_LIB" not in os.environ and _build.is_stale():
+        # sources newer than the library build() left: rebuild into a temporary directory, never into the tree (which
+        # may be read-only)
+        tmp = tempfile.mkdtemp(prefix="gnode_b200_")
+        atexit.register(shutil.rmtree, tmp, True)
+        os.environ["GNODE_B200_LIB"] = _build.build_library(force=True, out=os.path.join(tmp, "libgnode_b200.so"))
     L = _lib.lib()
 
     from gn_ode_sir_b200.parallel import shard_trials
@@ -399,13 +420,26 @@ def main():
     # points emitted into one reused [T, M_chunk, 3] buffer
     dev_sets = [hs.to(dev) for hs in host_sets]
     out_full = torch.empty((T, rows_full, 3), dtype=torch.float32, device=dev)
+    dump, dump_rows = None, None
+    if args.dump_outputs:
+        # per chunk: (row indices within the chunk, [T, rows, 3] destination) of the job-wide seeded sample
+        pick = np.random.default_rng(0).choice(total_trials * N, size=min(DUMP_ROWS, total_trials * N), replace=False)
+        dump_rows = np.sort(pick[(pick >= lo * N) & (pick < hi * N)])
+        dump = []
+        for c0, c1 in bounds:
+            sel = dump_rows[(dump_rows >= c0 * N) & (dump_rows < c1 * N)] - c0 * N
+            dump.append((torch.from_numpy(sel).to(dev), torch.empty((T, len(sel), 3), dtype=torch.float32, device=dev)))
 
-    def job_resident():
-        for (c0, c1), ds in zip(bounds, dev_sets):
+    def job_resident(capture=None):
+        for k, ((c0, c1), ds) in enumerate(zip(bounds, dev_sets)):
             if c1 - c0 == chunk:
                 blk.forward_trials(ds, None, None, probs_out=out_full, workspace=ws)
+                probs = out_full
             else:                                                      # ragged last chunk: its own (smaller) buffers
-                blk.forward_trials(ds, None, None)
+                probs = blk.forward_trials(ds, None, None)
+            if capture is not None:
+                probs = probs if probs is out_full else torch.cat(probs, -1)
+                torch.index_select(probs, 1, capture[k][0], out=capture[k][1])
 
     with torch.no_grad():
         for _ in range(args.warmup):
@@ -417,14 +451,20 @@ def main():
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
         barrier()
         ev[0].record()
-        for _ in range(args.steps):
-            job_resident()
+        for i in range(args.steps):
+            job_resident(dump if i == args.steps - 1 else None)
         ev[1].record()
         barrier()
         clocks = sampler.stop()
         launches = int(L.gnode_launch_count()) - launches0
         ms_local = ev[0].elapsed_time(ev[1])
         ms_total = max_over_ranks(ms_local)
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        suffix = "_rank%d" % rank if world > 1 else ""
+        np.save(os.path.join(args.dump_outputs, "probs_sample%s.npy" % suffix), torch.cat([d for _, d in dump], 1).cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, "probs_sample_rows%s.npy" % suffix), dump_rows.astype(np.float64))
+        del dump
     ms_per_step = ms_total / args.steps
     value = units_per_step / (ms_per_step * 1e-3)
     # dominant kernel = the fused Euler-step kernel: (T-1) launches per chunk, each over the chunk's rows; the trial

@@ -21,20 +21,20 @@ def _nvcc():
     raise RuntimeError("nvcc not found: libgnode_b200.so cannot be built")
 
 
-def is_stale():
-    if not os.path.exists(LIB_PATH):
+def is_stale(out=LIB_PATH):
+    if not os.path.exists(out):
         return True
-    t = os.path.getmtime(LIB_PATH)
+    t = os.path.getmtime(out)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)]
     deps.append(os.path.join(os.path.dirname(PKG_DIR), "include", "gnode_b200.h"))
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_library(force=False, extra_flags=(), verbose=False):
-    """Compile every .cu of the package for sm_100a into LIB_PATH. Returns LIB_PATH."""
-    if not force and not is_stale():
-        return LIB_PATH
-    cmd = [_nvcc()] + NVCC_FLAGS + list(extra_flags) + ["-o", LIB_PATH] + [os.path.join(CSRC, s) for s in SOURCES]
+def build_library(force=False, extra_flags=(), verbose=False, out=LIB_PATH):
+    """Compile every .cu of the package for sm_100a into `out` (default LIB_PATH). Returns `out`."""
+    if not force and not is_stale(out):
+        return out
+    cmd = [_nvcc()] + NVCC_FLAGS + list(extra_flags) + ["-o", out] + [os.path.join(CSRC, s) for s in SOURCES]
     if verbose:
         print(" ".join(cmd))
     res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
@@ -42,4 +42,4 @@ def build_library(force=False, extra_flags=(), verbose=False):
         raise RuntimeError("nvcc failed:\n" + res.stdout)
     if verbose and res.stdout:
         print(res.stdout)
-    return LIB_PATH
+    return out

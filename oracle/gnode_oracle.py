@@ -9,9 +9,8 @@ Parity status: the reference ships NO test, golden vector or known-answer for
 this path (SURVEY.md section 4), so this oracle is pinned the other way the
 task allows: against outputs of the reference's own classes executed in the
 build container (``oracle/ref_harness.py`` + ``tests/golden/make_golden.py``;
-``tests/test_oracle_vs_reference.py`` demands bit-equality on CPU fp32/fp64
-whenever ``/root/reference`` is present, and ``tests/test_oracle_golden.py``
-re-checks the committed fixtures everywhere).  The torchdiffeq boundary itself
+``tests/test_oracle_vs_reference.py`` and ``tests/test_oracle_golden.py``
+check the committed fixtures bit for bit).  The torchdiffeq boundary itself
 (un-vendored ``torchdiffeq==0.2.2``, requirements.txt:59) is restated from the
 published algorithm and is "parity unpinned" by any reference-held test.
 

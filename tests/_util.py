@@ -1,4 +1,5 @@
 """Shared helpers for the test-suite (golden fixture loading, oracle inputs)."""
+import contextlib
 import glob
 import os
 
@@ -13,6 +14,20 @@ GOLDEN_CASES = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(G
 # fp64 one by ~100 %): those cases are judged against the float64 run, err(ours) <= max(bar, 2 * err(reference fp32)).
 LARGE_CASES = [c for c in GOLDEN_CASES if any(k in c for k in ("fbsocial", "openflights", "wikivote", "train5"))]
 STRICT_CASES = [c for c in GOLDEN_CASES if c not in LARGE_CASES]
+# The fixtures were written with 8 intra-op threads. On CPU, torch splits elementwise ops (sigmoid) and GEMMs into
+# per-thread ranges, and where a range ends decides which elements take the vectorised path and which the scalar tail:
+# the fp32 results' last bits follow the thread count, so bit-exact comparisons with the fixtures run with 8 threads.
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    prev = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(prev)
 
 
 class Golden:
