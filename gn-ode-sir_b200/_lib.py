@@ -78,6 +78,10 @@ SIGNATURES = {
     "gnode_rollout_backward_aux": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(GnodeParams), c_int32,
                                            c_float_p, c_void_p, c_void_p, c_void_p, c_int32_p, c_int32, c_int32,
                                            c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gnode_rollout_backward_input": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(GnodeParams), c_int32,
+                                             c_float_p, c_void_p, c_void_p, c_void_p, c_int32_p, c_int32, c_int32,
+                                             c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "gnode_trials_grad": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "gnode_mc_sir_workspace_bytes": (c_size_t, [c_void_p, c_int32]),
     "gnode_mc_sir": (c_int, [c_void_p, c_void_p, c_int32, ctypes.c_float, ctypes.c_float, c_int32, c_int32,
                              ctypes.c_uint64, c_void_p, c_void_p, c_size_t, c_void_p]),

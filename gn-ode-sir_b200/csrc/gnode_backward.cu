@@ -38,6 +38,13 @@ constexpr int DEC_COUNT = 4 * H + 4 + 4 + 1;     // linear3.weight, linear3.bias
 constexpr int LIN_COUNT = H * H + H;             // odefunc.linear.weight, bias
 constexpr int ENC_COUNT = 2 * H;                 // linearS1.weight, bias
 
+// Sum over the 16 lanes of a half-warp, in a fixed order (all 32 lanes of the warp must call it).
+__device__ __forceinline__ float halfwarp_sum(float v) {
+#pragma unroll
+    for (int off = 8; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+    return v;
+}
+
 struct BwdArgs {
     GnBatchView bv;
     const float* x; int64_t ldx;   // beta = x[:,3], gamma = x[:,4]; encoder inputs x[:,0:3]
@@ -47,6 +54,7 @@ struct BwdArgs {
     float* Sp; float* Ip; float* AI; float* G;   // [M][H] scratch
     const float* Ipf; const float* AIf;          // [M][H] I'_j and AI_j = A I'_j kept by the forward (auxiliary storage), or null
     float* part;                   // per-block partial sums of this kernel family
+    float* gx; int64_t ldgx;       // dL/dx [M][ldgx] (columns 0..4) or null: no input gradient
     float dt;
     int only_dec;                  // 1: only a += D(y, gP)
     gnode_params_t p;
@@ -131,6 +139,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) bwd_transform_g_kernel(const BwdA
             const int idx = tid + i * NTHREADS;
             const int rr = idx >> 4, c4 = idx & 15;
             const int64_t g = tile0 + rr;
+            float gb = 0.f;
             if (g < M) {
                 const size_t off = (size_t)g * H + 4 * c4;
                 const float4 aS = ldg4(a.a + off), aI = ldg4(a.a + plane + off), ai = ldg4_stream(a.AIf + off);
@@ -147,6 +156,13 @@ __global__ void __launch_bounds__(NTHREADS, 2) bwd_transform_g_kernel(const BwdA
 #undef GN_G
                 stg4(a.G + off, G);
                 stg4(a.Sp + off, gz);
+                if (a.gx) gb = (aI.x - aS.x) * ai.x * sp.x + (aI.y - aS.y) * ai.y * sp.y +
+                               (aI.z - aS.z) * ai.z * sp.z + (aI.w - aS.w) * ai.w * sp.w;
+            }
+            // dL/dbeta of the row += dt * sum_h (aI - aS) AI S' (half-warp reduction; one lane per row adds)
+            if (a.gx) {
+                gb = halfwarp_sum(gb);
+                if (g < M && c4 == 0) a.gx[(size_t)g * a.ldgx + 3] += a.dt * gb;
             }
         }
         __syncthreads();
@@ -436,6 +452,24 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_gz_kernel(const BwdArgs a)
             if (!AUX) stg4(a.Sp + off, gzs);
             stg4(a.AI + off, gzi);
         }
+        // dL/dgamma of the row += dt * sum_h (aR - aI) I'; without auxiliary storage dL/dbeta += dt * sum_h (aI - aS) AI S'
+        // as well (with it, bwd_transform_g_kernel adds that term). Half-warp reductions, one lane per row adds.
+        if (a.gx) {
+            float sg = 0.f, sb = 0.f;
+            if (valid) {
+                sg = (aR.x - aI.x) * ip.x + (aR.y - aI.y) * ip.y + (aR.z - aI.z) * ip.z + (aR.w - aI.w) * ip.w;
+                if (!AUX)
+                    sb = (aI.x - aS.x) * ai.x * sp.x + (aI.y - aS.y) * ai.y * sp.y + (aI.z - aS.z) * ai.z * sp.z +
+                         (aI.w - aS.w) * ai.w * sp.w;
+            }
+            sg = halfwarp_sum(sg);
+            if (!AUX) sb = halfwarp_sum(sb);
+            if (valid && l == 0) {
+                float* gr = a.gx + (size_t)g * a.ldgx;
+                if (!AUX) gr[3] += a.dt * sb;
+                gr[4] += a.dt * sg;
+            }
+        }
     }
 }
 
@@ -609,6 +643,9 @@ constexpr int K3B_THREADS = 256;
 constexpr int K3B_SM_G = 0, K3B_SM_X = 32768, K3B_SM_WTHI = 65536, K3B_SM_WTLO = K3B_SM_WTHI + H * H * 4,
               K3B_SM_BAR = K3B_SM_WTLO + H * H * 4, K3B_SM_TOTAL = K3B_SM_BAR + 16 + 1024;
 
+// WGRAD = false: no parameter gradient wanted (input gradients only): the vW FFMA loop, the vb column sums and the fold
+// into the slots are compiled out; the state VJP and the adjoint's read-modify-write are the same instructions.
+template <bool WGRAD>
 __global__ void __launch_bounds__(K3B_THREADS, 2) bwd_vjp2_kernel(const BwdArgs a) {
     extern __shared__ unsigned char smem_raw[];
     unsigned char* smem = smem_raw + ((1024u - (umma::smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -684,7 +721,7 @@ __global__ void __launch_bounds__(K3B_THREADS, 2) bwd_vjp2_kernel(const BwdArgs 
             __syncthreads();
             // ---- vW[h][j] += sum_r gz[r][h] x[r][j] ; vb[h] += sum_r gz[r][h]   (fp32 FFMA)
 #pragma unroll 1
-            for (int r8 = 0; r8 < 8; ++r8) {
+            for (int r8 = 0; r8 < (WGRAD ? 8 : 0); ++r8) {      // (no trip without a parameter gradient)
                 const unsigned char* gp = Gb + r8 * 1024;
                 const unsigned char* xp = Xb + r8 * 1024;
 #pragma unroll
@@ -707,7 +744,7 @@ __global__ void __launch_bounds__(K3B_THREADS, 2) bwd_vjp2_kernel(const BwdArgs 
                 const int off = sw_off(idx >> 4, idx & 15);
                 float4 hi, lo;
                 const float4 gz = lds4(G, off);
-                gbv.x += gz.x; gbv.y += gz.y; gbv.z += gz.z; gbv.w += gz.w;
+                if (WGRAD) { gbv.x += gz.x; gbv.y += gz.y; gbv.z += gz.z; gbv.w += gz.w; }
                 umma::tf32_split4(gz, hi, lo);
                 sts4(G, off, hi); sts4(X, off, lo);
             }
@@ -746,7 +783,7 @@ __global__ void __launch_bounds__(K3B_THREADS, 2) bwd_vjp2_kernel(const BwdArgs 
     }
     // fold the two partial sums (row groups) of every output element: red[2][64][64] over the gz tile, red_b[16][64]
     // over the state tile (the tile loop has ended with a block barrier)
-    {
+    if (WGRAD) {
         float* red = reinterpret_cast<float*>(G);
         float* red_b = reinterpret_cast<float*>(X);
 #pragma unroll
@@ -775,26 +812,45 @@ __global__ void __launch_bounds__(K3B_THREADS, 2) bwd_vjp2_kernel(const BwdArgs 
 
 // ---------------------------------------------------------------- K4: encoder backward
 // y0 = relu(c * w1 + b1): d w1[h] = sum a0[h] [y0>0] c ; d b1[h] = sum a0[h] [y0>0]   (c in {S0,I0,R0})
+// Input gradient (a.gx): dL/dc = sum_h a0[h] [y0>0] w1[h], stored into columns 0..2. Parameter partials only when a.part.
 __global__ void __launch_bounds__(ROW_THREADS) bwd_encoder_kernel(const BwdArgs a) {
     __shared__ float red[ROW_THREADS / 16][16][9];
     const int tid = threadIdx.x, l = tid & 15, hw = tid >> 4;
     const int M = a.bv.M;
     const size_t plane = (size_t)M * H;
     float gw[4] = {0.f, 0.f, 0.f, 0.f}, gb[4] = {0.f, 0.f, 0.f, 0.f};
-    for (int64_t g = (int64_t)blockIdx.x * (ROW_THREADS / 16) + hw; g < M; g += (int64_t)gridDim.x * (ROW_THREADS / 16)) {
-        const size_t off = (size_t)g * H + 4 * l;
-        const float* xr = a.x + (size_t)g * a.ldx;
+    const float4 w1 = a.gx ? ldg4(a.p.s1_w + 4 * l) : make_float4(0.f, 0.f, 0.f, 0.f);
+    const int hw_per_grid = gridDim.x * (ROW_THREADS / 16);
+    const int64_t n_iter = (M + hw_per_grid - 1) / hw_per_grid;        // warp-uniform trip count (shuffles inside)
+    for (int64_t it = 0; it < n_iter; ++it) {
+        const int64_t g = it * hw_per_grid + (int64_t)blockIdx.x * (ROW_THREADS / 16) + hw;
+        const bool valid = g < M;
+        float gc[3] = {0.f, 0.f, 0.f};
+        if (valid) {
+            const size_t off = (size_t)g * H + 4 * l;
+            const float* xr = a.x + (size_t)g * a.ldx;
 #pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            const float c = xr[k];
-            const float4 y0 = ldg4_stream(a.y + k * plane + off);
-            const float4 av = ldg4_stream(a.a + k * plane + off);
-            const float m0 = y0.x > 0.f ? av.x : 0.f, m1 = y0.y > 0.f ? av.y : 0.f;
-            const float m2 = y0.z > 0.f ? av.z : 0.f, m3 = y0.w > 0.f ? av.w : 0.f;
-            gw[0] = fmaf(m0, c, gw[0]); gw[1] = fmaf(m1, c, gw[1]); gw[2] = fmaf(m2, c, gw[2]); gw[3] = fmaf(m3, c, gw[3]);
-            gb[0] += m0; gb[1] += m1; gb[2] += m2; gb[3] += m3;
+            for (int k = 0; k < 3; ++k) {
+                const float c = xr[k];
+                const float4 y0 = ldg4_stream(a.y + k * plane + off);
+                const float4 av = ldg4_stream(a.a + k * plane + off);
+                const float m0 = y0.x > 0.f ? av.x : 0.f, m1 = y0.y > 0.f ? av.y : 0.f;
+                const float m2 = y0.z > 0.f ? av.z : 0.f, m3 = y0.w > 0.f ? av.w : 0.f;
+                gw[0] = fmaf(m0, c, gw[0]); gw[1] = fmaf(m1, c, gw[1]); gw[2] = fmaf(m2, c, gw[2]); gw[3] = fmaf(m3, c, gw[3]);
+                gb[0] += m0; gb[1] += m1; gb[2] += m2; gb[3] += m3;
+                gc[k] = m0 * w1.x + m1 * w1.y + m2 * w1.z + m3 * w1.w;
+            }
+        }
+        if (a.gx) {
+#pragma unroll
+            for (int k = 0; k < 3; ++k) gc[k] = halfwarp_sum(gc[k]);
+            if (valid && l == 0) {
+                float* gr = a.gx + (size_t)g * a.ldgx;
+                gr[0] = gc[0]; gr[1] = gc[1]; gr[2] = gc[2];
+            }
         }
     }
+    if (!a.part) return;                                       // no parameter gradient wanted
 #pragma unroll
     for (int i = 0; i < 4; ++i) { red[hw][l][i] = gw[i]; red[hw][l][4 + i] = gb[i]; }
     __syncthreads();
@@ -816,6 +872,30 @@ __global__ void reduce_partials_kernel(const float* __restrict__ part, int n_slo
     out[i] = s;
 }
 
+// Per-instance sums of grad_x columns 3 and 4 (the gradient of compact descriptors' beta[i], gamma[i]): one CTA per
+// instance, every thread sums a fixed strided subset of the rows in row order, then a fixed-shape tree (no atomics).
+constexpr int TG_THREADS = 256;
+__global__ void __launch_bounds__(TG_THREADS) trials_grad_kernel(const GnBatchView bv, const float* __restrict__ gx,
+                                                                 int64_t ldgx, float* __restrict__ gbeta,
+                                                                 float* __restrict__ ggamma) {
+    __shared__ float sb[TG_THREADS], sg[TG_THREADS];
+    const int tid = threadIdx.x;
+    const GnInstance I = bv.inst[blockIdx.x];
+    float b = 0.f, g = 0.f;
+    for (int n = tid; n < I.n; n += TG_THREADS) {
+        const float* r = gx + (size_t)(I.row0 + n) * ldgx;
+        b += r[3]; g += r[4];
+    }
+    sb[tid] = b; sg[tid] = g;
+    __syncthreads();
+#pragma unroll
+    for (int w = TG_THREADS / 2; w >= 1; w >>= 1) {
+        if (tid < w) { sb[tid] += sb[tid + w]; sg[tid] += sg[tid + w]; }
+        __syncthreads();
+    }
+    if (tid == 0) { gbeta[blockIdx.x] = sb[0]; ggamma[blockIdx.x] = sg[0]; }
+}
+
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // 2 (default) = bwd_vjp2_kernel (two 256-thread CTAs per SM, parts in sequence), 1 = bwd_vjp_kernel; env GNODE_BWD_VJP.
@@ -832,10 +912,13 @@ static int vjp_kernel_choice() {
     }
     return g_vjp_kernel;
 }
-static int launch_vjp(const BwdArgs& a, int grid, cudaStream_t stream) {
+static int launch_vjp(const BwdArgs& a, int grid, bool wgrad, cudaStream_t stream) {
     switch (vjp_kernel_choice()) {
-        case 1: bwd_vjp_kernel<<<grid, NTHREADS, K3_SM_TOTAL, stream>>>(a); break;
-        default: bwd_vjp2_kernel<<<grid, K3B_THREADS, K3B_SM_TOTAL, stream>>>(a); break;
+        case 1: bwd_vjp_kernel<<<grid, NTHREADS, K3_SM_TOTAL, stream>>>(a); break;   // (computes its partials anyway)
+        default:
+            if (wgrad) bwd_vjp2_kernel<true><<<grid, K3B_THREADS, K3B_SM_TOTAL, stream>>>(a);
+            else bwd_vjp2_kernel<false><<<grid, K3B_THREADS, K3B_SM_TOTAL, stream>>>(a);
+            break;
     }
     GN_LAUNCH_CHECK();
     return GNODE_OK;
@@ -903,11 +986,22 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
                                           const float* grad_probs, const int32_t* out_steps, int32_t n_out,
                                           int32_t grad_mode, float* grads_out, void* workspace, size_t workspace_bytes,
                                           void* stream_) {
-    if (!b || !x || !p || !traj || !grad_probs || !grads_out || !workspace || T < 1 || ldx < 5 ||
-        (T > 1 && !dt_host) || (grad_mode != GNODE_GRAD_ADJOINT && grad_mode != GNODE_GRAD_DISCRETE)) {
-        set_error("gnode_rollout_backward: bad arguments (T=%d ldx=%lld grad_mode=%d)", T, (long long)ldx, grad_mode);
+    return gnode_rollout_backward_input(b, x, ldx, p, T, dt_host, traj, aux, grad_probs, out_steps, n_out, grad_mode,
+                                        grads_out, nullptr, 0, workspace, workspace_bytes, stream_);
+}
+
+extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p,
+                                            int32_t T, const float* dt_host, const float* traj, const float* aux,
+                                            const float* grad_probs, const int32_t* out_steps, int32_t n_out,
+                                            int32_t grad_mode, float* grads_out, float* grad_x, int64_t ldgx,
+                                            void* workspace, size_t workspace_bytes, void* stream_) {
+    if (!b || !x || !p || !traj || !grad_probs || (!grads_out && !grad_x) || (grad_x && ldgx < 5) || !workspace ||
+        T < 1 || ldx < 5 || (T > 1 && !dt_host) || (grad_mode != GNODE_GRAD_ADJOINT && grad_mode != GNODE_GRAD_DISCRETE)) {
+        set_error("gnode_rollout_backward: bad arguments (T=%d ldx=%lld ldgx=%lld grad_mode=%d grads_out=%p grad_x=%p)", T,
+                  (long long)ldx, (long long)ldgx, grad_mode, (void*)grads_out, (void*)grad_x);
         return GNODE_ERR_ARG;
     }
+    const bool wgrad = grads_out != nullptr;
     OutSel sel;
     int rc = make_out_sel(T, out_steps, n_out, &sel, "gnode_rollout_backward_sel");
     if (rc) return rc;
@@ -923,7 +1017,8 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
         GN_CUDA(cudaFuncSetAttribute(bwd_transform_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, K1_SM_TOTAL));
         GN_CUDA(cudaFuncSetAttribute(bwd_transform_g_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, K1_SM_TOTAL));
         GN_CUDA(cudaFuncSetAttribute(bwd_vjp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, K3_SM_TOTAL));
-        GN_CUDA(cudaFuncSetAttribute(bwd_vjp2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, K3B_SM_TOTAL));
+        GN_CUDA(cudaFuncSetAttribute(bwd_vjp2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K3B_SM_TOTAL));
+        GN_CUDA(cudaFuncSetAttribute(bwd_vjp2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K3B_SM_TOTAL));
         configured[b->device & 63] = true;
     }
     const size_t M = (size_t)b->M;
@@ -944,8 +1039,10 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
                 if (key == 0) key = 1469598103934665603ull;
                 for (size_t i = 0; i < n; ++i) { key ^= c[i]; key *= 1099511628211ull; }
             };
-            const void* ptrs[] = {x, traj, aux, grad_probs, grads_out, workspace, stream_};
+            // (grads_out == NULL, i.e. no parameter gradient, and grad_x == NULL are part of the pointers)
+            const void* ptrs[] = {x, traj, aux, grad_probs, grads_out, workspace, stream_, grad_x};
             mix(ptrs, sizeof(ptrs)); mix(p, sizeof(*p)); mix(&ldx, sizeof(ldx)); mix(&T, sizeof(T));
+            mix(&ldgx, sizeof(ldgx));
             mix(&grad_mode, sizeof(grad_mode)); mix(dt_host, sizeof(float) * (size_t)(T > 1 ? T - 1 : 0));
             mix(sel.slot.data(), sizeof(int) * sel.slot.size());
             const int vk = vjp_kernel_choice();
@@ -975,6 +1072,7 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
     BwdArgs a;
     a.bv = gn_view(b);
     a.x = x; a.ldx = ldx; a.p = *p;
+    a.gx = grad_x; a.ldgx = ldgx;
     a.a = (float*)(ws + pl.off_a);
     a.Sp = (float*)(ws + pl.off_sp); a.Ip = (float*)(ws + pl.off_ip);
     a.AI = (float*)(ws + pl.off_ai); a.G = (float*)(ws + pl.off_g);
@@ -984,6 +1082,8 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
     // adjoint and partial-sum slots start at zero
     GN_CUDA(cudaMemsetAsync(ws + pl.off_a, 0, 3 * M * H * sizeof(float), stream));
     GN_CUDA(cudaMemsetAsync(ws + pl.off_pdec, 0, pl.off_penc - pl.off_pdec, stream));
+    // dL/dbeta, dL/dgamma are sums over the reverse steps (columns 3, 4 of grad_x); the encoder stores columns 0..2
+    if (grad_x) GN_CUDA(cudaMemset2DAsync(grad_x + 3, (size_t)ldgx * sizeof(float), 0, 2 * sizeof(float), M, stream));
 
     auto state = [&](int j) { return traj + (size_t)j * 3 * M * H; };
     // cotangent of grid point j, or null when its probabilities were not emitted (sparse dL/dprobs: the loss of the
@@ -1010,7 +1110,7 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
             bwd_gz_kernel<true><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
             GN_LAUNCH_CHECK();
             a.part = plin;
-            return launch_vjp(a, pl.grid_tile3, stream);
+            return launch_vjp(a, pl.grid_tile3, wgrad, stream);
         }
         a.y = state(j); a.gP = with_decoder ? gp(j) : nullptr; a.dt = dt; a.only_dec = 0;
         a.part = nullptr;
@@ -1023,7 +1123,7 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
         bwd_gz_kernel<false><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
         GN_LAUNCH_CHECK();
         a.part = plin;
-        return launch_vjp(a, pl.grid_tile3, stream);
+        return launch_vjp(a, pl.grid_tile3, wgrad, stream);
     };
     int jmax = T - 1;                             // last grid point with a cotangent: the adjoint is zero beyond it
     while (jmax > 0 && sel.slot[jmax] < 0) --jmax;
@@ -1039,9 +1139,11 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
             if ((rc = dec_only(j))) return rc;
         }
     }
-    a.y = state(0); a.part = penc;
+    a.y = state(0); a.part = wgrad ? penc : nullptr;
     bwd_encoder_kernel<<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
     GN_LAUNCH_CHECK();
+    // (without a parameter gradient the decoder kernels' partial sums are left unread in their slots)
+    if (!wgrad) return GNODE_OK;
     // fold the per-block slots into the flat gradient vector (layout of include/gnode_b200.h)
     reduce_partials_kernel<<<(LIN_COUNT + 255) / 256, 256, 0, stream>>>(plin, pl.grid_tile3, LIN_COUNT,
                                                                         grads_out + GNODE_GRAD_OFF_LIN_W);
@@ -1074,5 +1176,19 @@ extern "C" int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64
     b->bwd_graphs.push_back({key, (void*)exec, kernels});
     GN_CUDA(cudaGraphLaunch(exec, user_stream));
     (void)use_graph;
+    return GNODE_OK;
+}
+
+extern "C" int gnode_trials_grad(gnode_batch_t b, const float* grad_x, int64_t ldgx, float* grad_beta, float* grad_gamma,
+                                 void* stream_) {
+    if (!b || !grad_x || ldgx < 5 || !grad_beta || !grad_gamma) {
+        set_error("gnode_trials_grad: bad arguments (ldgx=%lld)", (long long)ldgx);
+        return GNODE_ERR_ARG;
+    }
+    int rc = check_current_device(b, "gnode_trials_grad");
+    if (rc) return rc;
+    if (b->n_inst == 0) return GNODE_OK;
+    trials_grad_kernel<<<b->n_inst, TG_THREADS, 0, (cudaStream_t)stream_>>>(gn_view(b), grad_x, ldgx, grad_beta, grad_gamma);
+    GN_LAUNCH_CHECK();
     return GNODE_OK;
 }

@@ -118,8 +118,10 @@ class ODEBlock(nn.Module):
 
     def forward_trials(self, instances, seeds, beta, gamma, out_steps=None):
         """Rollout from compact descriptors (N4): instance i runs on graph instances[i] with seeds[i], beta[i], gamma[i]
-        (replaces the dense per-instance blocks of ode_nn_ngraphs.py:326-345). Returns (S, I, R)."""
+        (replaces the dense per-instance blocks of ode_nn_ngraphs.py:326-345). Returns (S, I, R). beta / gamma given as
+        tensors that require grad receive dL/dbeta[i], dL/dgamma[i]."""
         batch = self.odefunc.batch_from_instances(instances)
         trials = _ro.TrialSet(seeds, beta, gamma, batch.sizes, self.linearS1.weight.device)
-        probs = self._finish(_ro.rollout_trials(batch, trials, self._dt, self._params(), self.grad_mode, out_steps))
+        probs = self._finish(_ro.rollout_trials(batch, trials, self._dt, self._params(), self.grad_mode, out_steps,
+                                                beta=beta, gamma=gamma))
         return probs.chunk(3, dim=-1)

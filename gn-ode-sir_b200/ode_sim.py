@@ -109,11 +109,12 @@ class ODEBlock(nn.Module):
     def forward_trials(self, seeds, beta, gamma, out_steps=None, probs_out=None, workspace=None):
         """The same rollout from compact trial descriptors (N4): seeds[i] = node ids infected at t = 0 in trial i,
         beta[i], gamma[i] -- instead of the dense [N, 3+H] block per trial main() builds (ode_nn_ngraph_sim.py:371-390).
-        Returns (S, I, R), each [T (or len(out_steps)), B*N, 1]."""
+        Returns (S, I, R), each [T (or len(out_steps)), B*N, 1]. beta / gamma given as tensors that require grad receive
+        dL/dbeta[i], dL/dgamma[i] (calibration of a trial through the trained model)."""
         is_set = isinstance(seeds, _ro.TrialSet)                      # a prepared (device-resident) descriptor set
         batch = self.odefunc.batch_for(seeds.n_inst if is_set else len(seeds))
         dev = self.linearS1.weight.device
         trials = seeds if is_set else _ro.TrialSet(seeds, beta, gamma, batch.sizes, dev)
         probs = self._finish(_ro.rollout_trials(batch, trials, self._dt, self._params(), self.grad_mode, out_steps,
-                                                probs_out, workspace))
+                                                probs_out, workspace, *((None, None) if is_set else (beta, gamma))))
         return probs.chunk(3, dim=-1)

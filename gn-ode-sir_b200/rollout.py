@@ -106,7 +106,7 @@ class _Rollout(torch.autograd.Function):
             _check_cuda_f32(p, k)
             ps.append(p.detach().contiguous())
         # grad mode is always off inside forward(): the caller's grad mode arrives as `want_grad`
-        need_grad = bool(want_grad) and any(ctx.needs_input_grad[6:])
+        need_grad = bool(want_grad) and (ctx.needs_input_grad[0] or any(ctx.needs_input_grad[6:]))
         with torch.cuda.device(x.device):
             traj = torch.empty((T, 3, M, H), dtype=torch.float32, device=x.device) if need_grad else None
             probs = torch.empty((n_out, M, 3), dtype=torch.float32, device=x.device)
@@ -131,6 +131,7 @@ class _Rollout(torch.autograd.Function):
             ctx.save_for_backward(x, traj, *ps)
             ctx.batch, ctx.dt, ctx.grad_mode, ctx.steps = batch, dt, grad_mode, steps
             ctx.aux = aux if filled.value == 1 else None
+            ctx.wgrad = any(ctx.needs_input_grad[6:])       # False: input gradients only (no weight-gradient phase)
         return probs
 
     @staticmethod
@@ -144,31 +145,37 @@ class _Rollout(torch.autograd.Function):
         steps = ctx.steps
         steps_p = steps.ctypes.data_as(_lib.c_int32_p) if steps is not None else None
         with torch.cuda.device(x.device):
-            grads = torch.empty(_lib.GRAD_COUNT, dtype=torch.float32, device=x.device)
+            grads = torch.empty(_lib.GRAD_COUNT, dtype=torch.float32, device=x.device) if ctx.wgrad else None
+            # dL/dx: columns 0..4 written by the sweep, the others (graph marker, unused bg channels) carry no gradient
+            grad_x = torch.zeros(tuple(x.shape), dtype=torch.float32, device=x.device) if ctx.needs_input_grad[0] else None
             ws_bytes = int(L.gnode_backward_workspace_bytes(batch.handle))
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
             pstruct = _params_struct(ps)
             mode = {"adjoint": _lib.GRAD_ADJOINT, "discrete": _lib.GRAD_DISCRETE}[ctx.grad_mode]
-            _lib.check(L.gnode_rollout_backward_aux(batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T,
-                                                    dt.ctypes.data_as(_lib.c_float_p), _ptr(traj),
-                                                    _ptr(ctx.aux) if ctx.aux is not None else None, _ptr(grad_probs),
-                                                    steps_p, len(steps) if steps is not None else 0, mode,
-                                                    _ptr(grads), _ptr(ws), ws_bytes, _stream(x.device)),
-                       "gnode_rollout_backward_aux")
+            _lib.check(L.gnode_rollout_backward_input(batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T,
+                                                      dt.ctypes.data_as(_lib.c_float_p), _ptr(traj),
+                                                      _ptr(ctx.aux) if ctx.aux is not None else None, _ptr(grad_probs),
+                                                      steps_p, len(steps) if steps is not None else 0, mode,
+                                                      _ptr(grads) if grads is not None else None,
+                                                      _ptr(grad_x) if grad_x is not None else None,
+                                                      grad_x.stride(0) if grad_x is not None else 0,
+                                                      _ptr(ws), ws_bytes, _stream(x.device)),
+                       "gnode_rollout_backward_input")
         out, off = [], 0
         for i, (k, shape) in enumerate(_lib.GRAD_LAYOUT):
             n = int(np.prod(shape))
             out.append(grads[off:off + n].view(shape) if ctx.needs_input_grad[6 + i] else None)
             off += n
-        return (None, None, None, None, None, None, *out)
+        return (grad_x, None, None, None, None, None, *out)
 
 
 def rollout(x, batch, dt, params, grad_mode="adjoint", out_steps=None):
     """x [M, >=5] -> probabilities [T, M, 3] (or [len(out_steps), M, 3]: only those grid points are decoded and
-    stored); params in PARAM_ORDER (state_dict names)."""
+    stored); params in PARAM_ORDER (state_dict names). Differentiable with respect to the parameters and to x (columns
+    S0, I0, R0, beta, gamma; the other columns get zero gradients)."""
     if grad_mode not in ("adjoint", "discrete"):
         raise ValueError("grad_mode must be 'adjoint' or 'discrete'")
-    want_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+    want_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
     return _Rollout.apply(x, batch, dt, grad_mode, want_grad, out_steps, *params)
 
 
@@ -176,7 +183,8 @@ class TrialSet:
     """Compact trial descriptors of one batch (N4): per instance the seed list (instance-local node ids), beta and
     gamma -- what main() expands into a dense [N, 3+H] block per trial on the host (ode_nn_ngraph_sim.py:371-390).
     A few KB per batch instead of 268 B per row. device=None keeps the set in pinned host memory (a dataset of
-    batches that a streaming loop copies into a device-resident set with copy_from)."""
+    batches that a streaming loop copies into a device-resident set with copy_from). beta and gamma may be sequences or
+    torch tensors; the set keeps detached copies (gradients reach them through rollout_trials' beta / gamma)."""
 
     def __init__(self, seeds, beta, gamma, sizes, device=None):
         if not (len(seeds) == len(beta) == len(gamma) == len(sizes)):
@@ -191,8 +199,9 @@ class TrialSet:
             ptr[i + 1] = ptr[i] + len(sd)
         self.n_inst = len(seeds)
         hi = torch.from_numpy(np.concatenate([ptr] + flat))
-        hf = torch.from_numpy(np.concatenate([np.asarray(beta, dtype=np.float32).reshape(-1),
-                                              np.asarray(gamma, dtype=np.float32).reshape(-1)]))
+        host = lambda v: v.detach().to("cpu", torch.float32).numpy() if torch.is_tensor(v) else v
+        hf = torch.from_numpy(np.concatenate([np.asarray(host(beta), dtype=np.float32).reshape(-1),
+                                              np.asarray(host(gamma), dtype=np.float32).reshape(-1)]))
         if torch.cuda.is_available():
             hi, hf = hi.pin_memory(), hf.pin_memory()
         self._host = (hi, hf)
@@ -237,13 +246,48 @@ def expand_trials(batch, trials, ldx=_lib.GNODE_TRIAL_LDX):
     return x
 
 
-def rollout_trials(batch, trials, dt, params, grad_mode="adjoint", out_steps=None, probs_out=None, workspace=None):
+class _ExpandTrials(torch.autograd.Function):
+    """expand_trials as a function of the descriptors' beta and gamma: dL/dbeta[i] and dL/dgamma[i] are the sums of
+    dL/dx[:, 3] and dL/dx[:, 4] over the rows of instance i (gnode_trials_grad, fixed summation order)."""
+
+    @staticmethod
+    def forward(ctx, beta, gamma, batch, trials):
+        ctx.batch = batch
+        ctx.meta = [(t.shape, t.dtype, t.device) for t in (beta, gamma)]
+        return expand_trials(batch, trials)
+
+    @staticmethod
+    def backward(ctx, gx):
+        L = _lib.lib()
+        gx = gx.contiguous()
+        n = len(ctx.batch.sizes)
+        with torch.cuda.device(gx.device):
+            gbg = torch.empty((2, n), dtype=torch.float32, device=gx.device)
+            _lib.check(L.gnode_trials_grad(ctx.batch.handle, _ptr(gx), gx.stride(0), _ptr(gbg[0]), _ptr(gbg[1]),
+                                           _stream(gx.device)), "gnode_trials_grad")
+        out = [g.reshape(shape).to(device=dev, dtype=dtype) for g, (shape, dtype, dev) in zip(gbg, ctx.meta)]
+        return out[0], out[1], None, None
+
+
+def rollout_trials(batch, trials, dt, params, grad_mode="adjoint", out_steps=None, probs_out=None, workspace=None,
+                   beta=None, gamma=None):
     """Rollout straight from compact trial descriptors. Without gradients: ONE C-ABI call (expansion into the
     workspace + rollout), optionally into caller-owned `probs_out` / `workspace` buffers (streaming loops reuse them).
-    With gradients: the compact x is kept for the reverse sweep."""
-    want_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+    With gradients: the compact x is kept for the reverse sweep. `beta` / `gamma`: the tensors the set was made from;
+    when one of them requires grad, it receives dL/dbeta[i] (dL/dgamma[i]) per instance. Seed sets are discrete and
+    have no gradient."""
+    want_x = torch.is_grad_enabled() and any(torch.is_tensor(v) and v.requires_grad for v in (beta, gamma))
+    want_grad = want_x or (torch.is_grad_enabled() and any(p.requires_grad for p in params))
     if want_grad:
-        return rollout(expand_trials(batch, trials), batch, dt, params, grad_mode, out_steps)
+        if want_x:
+            bt = beta if torch.is_tensor(beta) else trials.beta
+            gt = gamma if torch.is_tensor(gamma) else trials.gamma
+            if bt.numel() != trials.n_inst or gt.numel() != trials.n_inst:
+                raise ValueError("beta and gamma must hold one value per instance (%d)" % trials.n_inst)
+            x = _ExpandTrials.apply(bt, gt, batch, trials)
+        else:
+            x = expand_trials(batch, trials)
+        return rollout(x, batch, dt, params, grad_mode, out_steps)
     L = _lib.lib()
     if trials.n_inst != len(batch.sizes):
         raise ValueError("%d trial descriptors for a batch of %d instances" % (trials.n_inst, len(batch.sizes)))

@@ -236,6 +236,30 @@ int gnode_rollout_backward_aux(gnode_batch_t b, const float* x, int64_t ldx, con
                                const float* grad_probs, const int32_t* out_steps, int32_t n_out, int32_t grad_mode,
                                float* grads_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- input gradients: dL/d{S0, I0, R0, beta, gamma} -------------------------------
+ * The reference's autograd reaches every input column that enters the computation: S0, I0, R0 through the encoder
+ * relu(linearS1(c)) (ode_nn_ngraph_sim.py:151-156), beta and gamma through the bg block of the ODE state, which f reads
+ * (:60) and whose adjoint builds up over torchdiffeq's reverse sweep. Per reverse step at state y_j with cotangent
+ * a = (aS, aI, aR) and step dt (the same state and dt as the parameter VJP; ADJOINT: y_i with a_i, DISCRETE: exact
+ * back-propagation of the Euler loop):
+ *   dL/dbeta[r]  += dt * sum_h (aI - aS) AI S'       dL/dgamma[r] += dt * sum_h (aR - aI) I'
+ * and after the sweep, with the final adjoint a_0 and y_0 = relu(c w1 + b1):  dL/dc[r] = sum_h a0[r,h] [y0 > 0] w1[h].
+ * Reverse sweep with optional parameter and input gradients.
+ *   grads_out  [GNODE_GRAD_COUNT] or NULL: no parameter gradient (the weight-gradient phase is skipped)
+ *   grad_x     [M, ldgx] or NULL (ldgx >= 5): columns 0..4 overwritten with dL/d{S0, I0, R0, beta, gamma}, other
+ *              columns untouched; at least one of grads_out / grad_x non-NULL.
+ * grad_x == NULL is gnode_rollout_backward_aux, bit for bit. Same workspace (gnode_backward_workspace_bytes). Every row's
+ * gradient is summed in a fixed order without atomics: bitwise reproducible. */
+int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p, int32_t T,
+                                 const float* dt_host, const float* traj, const float* aux, const float* grad_probs,
+                                 const int32_t* out_steps, int32_t n_out, int32_t grad_mode, float* grads_out,
+                                 float* grad_x, int64_t ldgx, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Per-instance sums of grad_x columns 3 and 4 (instance i = rows [row0_i, row0_i + n_i)), in a fixed order:
+ * the gradient of compact trial descriptors' beta[i], gamma[i] (N4). grad_beta, grad_gamma: DEVICE float[n_inst]. */
+int gnode_trials_grad(gnode_batch_t b, const float* grad_x, int64_t ldgx, float* grad_beta, float* grad_gamma,
+                      void* stream);
+
 /* ---- N1: L1 loss on the sub-sampled prediction and its cotangent, fused -------
  * Replaces, per mini-batch, get_sir_t_nodes_torch x3 (60 row copies device -> CPU tensor, ode_nn.py:257-259), the
  * cat / transpose / .to(device) and nn.L1Loss on [:,1:,:] (ode_nn_ngraph_sim.py:230-234, ode_nn_ngraphs.py:216-220),
