@@ -21,6 +21,7 @@
 //   K2 bwd_row_kernel       : AI = A I' ; a += D(y_j,gP_j) (adjoint mode) ; gAI   -> AI, G, a
 //                             (discrete mode adds D in a separate row pass after K3)
 //   K3a bwd_gz_kernel      : A^T gAI, gz* (in place over Sp / AI)
+//   K3e bwd_edge_kernel    : dL/dw_rc += dt * gAI[r] . I'[c] per stored entry of A (only when edge gradients are asked)
 //   K3 bwd_vjp_kernel       : per-CTA vW / vb (FFMA), v = gz W into a (tcgen05)
 // Parameter-gradient partial sums live in per-CTA slots (no atomics: bitwise reproducible) and are
 // folded by reduce_partials_kernel at the end.
@@ -469,6 +470,64 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_gz_kernel(const BwdArgs a)
                 if (!AUX) gr[3] += a.dt * sb;
                 gr[4] += a.dt * sg;
             }
+        }
+    }
+}
+
+// ---------------------------------------------------------------- K3e: edge gradient (only when asked for)
+// The forward's neighbour sum is AI[r] = sum_c w_rc I'[c] at w = 1, so per reverse step, at the same state and dt as the
+// parameter VJP:   dL/dw_rc += dt * sum_h gAI[r,h] I'[c,h]   for every stored entry (r, c) of A.
+// Row kernel over the forward CSR (not the transpose): a half-warp holds G[r] = gAI (4 channels per lane) and loads 8
+// neighbour rows of I' per memory round trip, as gather_row does. Each edge's dot product is summed in a fixed order
+// (lane partials, then the 16-lane butterfly) and one lane per edge adds it into ge: no atomics, bitwise reproducible.
+// Launched after bwd_gz_kernel (which overwrites only Sp and AI: G and I' are intact) and before the tile kernel.
+// Ipr: I' of the step (the forward's auxiliary storage, or the Ip scratch); inst_e0[i]: first entry of instance i in ge.
+__global__ void __launch_bounds__(ROW_THREADS, 3) bwd_edge_kernel(const BwdArgs a, const float* __restrict__ Ipr,
+                                                                   const int64_t* __restrict__ inst_e0,
+                                                                   float* __restrict__ ge) {
+    const int tid = threadIdx.x, lane = tid & 31, l = tid & 15, hw = tid >> 4;
+    const int M = a.bv.M;
+    const int hw_per_grid = gridDim.x * (ROW_THREADS / 16);
+    const int64_t n_iter = (M + hw_per_grid - 1) / hw_per_grid;        // warp-uniform trip count (shuffles inside)
+    for (int64_t it = 0; it < n_iter; ++it) {
+        const int64_t g = it * hw_per_grid + (int64_t)blockIdx.x * (ROW_THREADS / 16) + hw;
+        const bool valid = g < M;
+        int row0 = 0, e0 = 0, deg = 0;
+        const int32_t* ci = nullptr;
+        float* out = nullptr;
+        float4 gr = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (valid) {
+            gr = ldg4(a.G + (size_t)g * H + 4 * l);
+            int inst = a.bv.tile_inst[g / TILE];
+            while (inst + 1 < a.bv.n_inst && a.bv.inst[inst + 1].row0 <= g) ++inst;
+            const GnInstance I = a.bv.inst[inst];
+            row0 = I.row0; ci = I.colidx;
+            const int n = (int)(g - row0);
+            e0 = I.rowptr[n];
+            deg = I.rowptr[n + 1] - e0;
+            out = ge + inst_e0[inst] + e0;
+        }
+        const int degmax = max(deg, __shfl_xor_sync(0xffffffffu, deg, 16));
+        for (int eb = 0; eb < degmax; eb += 16) {
+            const int mine = (eb + l < deg) ? ci[e0 + eb + l] + row0 : -1;
+            float res = 0.f;                                   // dot product of edge eb + l
+#pragma unroll
+            for (int jb = 0; jb < 16; jb += 8) {
+                if (eb + jb < degmax) {
+                    float4 v[8];
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const int c = __shfl_sync(0xffffffffu, mine, (lane & 16) + jb + j);
+                        v[j] = (c >= 0) ? ldg4(Ipr + (size_t)c * H + 4 * l) : make_float4(0.f, 0.f, 0.f, 0.f);
+                    }
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const float s = halfwarp_sum(dot4(gr, v[j]));
+                        if (l == jb + j) res = s;
+                    }
+                }
+            }
+            if (eb + l < deg) out[eb + l] += a.dt * res;
         }
     }
 }
@@ -995,10 +1054,21 @@ extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int
                                             const float* grad_probs, const int32_t* out_steps, int32_t n_out,
                                             int32_t grad_mode, float* grads_out, float* grad_x, int64_t ldgx,
                                             void* workspace, size_t workspace_bytes, void* stream_) {
-    if (!b || !x || !p || !traj || !grad_probs || (!grads_out && !grad_x) || (grad_x && ldgx < 5) || !workspace ||
-        T < 1 || ldx < 5 || (T > 1 && !dt_host) || (grad_mode != GNODE_GRAD_ADJOINT && grad_mode != GNODE_GRAD_DISCRETE)) {
-        set_error("gnode_rollout_backward: bad arguments (T=%d ldx=%lld ldgx=%lld grad_mode=%d grads_out=%p grad_x=%p)", T,
-                  (long long)ldx, (long long)ldgx, grad_mode, (void*)grads_out, (void*)grad_x);
+    return gnode_rollout_backward_edges(b, x, ldx, p, T, dt_host, traj, aux, grad_probs, out_steps, n_out, grad_mode,
+                                        grads_out, grad_x, ldgx, nullptr, workspace, workspace_bytes, stream_);
+}
+
+extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p,
+                                            int32_t T, const float* dt_host, const float* traj, const float* aux,
+                                            const float* grad_probs, const int32_t* out_steps, int32_t n_out,
+                                            int32_t grad_mode, float* grads_out, float* grad_x, int64_t ldgx,
+                                            float* grad_edge, void* workspace, size_t workspace_bytes, void* stream_) {
+    if (!b || !x || !p || !traj || !grad_probs || (!grads_out && !grad_x && !grad_edge) || (grad_x && ldgx < 5) ||
+        !workspace || T < 1 || ldx < 5 || (T > 1 && !dt_host) ||
+        (grad_mode != GNODE_GRAD_ADJOINT && grad_mode != GNODE_GRAD_DISCRETE)) {
+        set_error("gnode_rollout_backward: bad arguments (T=%d ldx=%lld ldgx=%lld grad_mode=%d grads_out=%p grad_x=%p "
+                  "grad_edge=%p)", T, (long long)ldx, (long long)ldgx, grad_mode, (void*)grads_out, (void*)grad_x,
+                  (void*)grad_edge);
         return GNODE_ERR_ARG;
     }
     const bool wgrad = grads_out != nullptr;
@@ -1039,8 +1109,8 @@ extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int
                 if (key == 0) key = 1469598103934665603ull;
                 for (size_t i = 0; i < n; ++i) { key ^= c[i]; key *= 1099511628211ull; }
             };
-            // (grads_out == NULL, i.e. no parameter gradient, and grad_x == NULL are part of the pointers)
-            const void* ptrs[] = {x, traj, aux, grad_probs, grads_out, workspace, stream_, grad_x};
+            // (grads_out == NULL, i.e. no parameter gradient, grad_x == NULL and grad_edge == NULL are part of the pointers)
+            const void* ptrs[] = {x, traj, aux, grad_probs, grads_out, workspace, stream_, grad_x, grad_edge};
             mix(ptrs, sizeof(ptrs)); mix(p, sizeof(*p)); mix(&ldx, sizeof(ldx)); mix(&T, sizeof(T));
             mix(&ldgx, sizeof(ldgx));
             mix(&grad_mode, sizeof(grad_mode)); mix(dt_host, sizeof(float) * (size_t)(T > 1 ? T - 1 : 0));
@@ -1084,6 +1154,15 @@ extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int
     GN_CUDA(cudaMemsetAsync(ws + pl.off_pdec, 0, pl.off_penc - pl.off_pdec, stream));
     // dL/dbeta, dL/dgamma are sums over the reverse steps (columns 3, 4 of grad_x); the encoder stores columns 0..2
     if (grad_x) GN_CUDA(cudaMemset2DAsync(grad_x + 3, (size_t)ldgx * sizeof(float), 0, 2 * sizeof(float), M, stream));
+    // dL/dw is a sum over the reverse steps as well (steps without an adjoint add nothing)
+    if (grad_edge && b->nnz_total > 0)
+        GN_CUDA(cudaMemsetAsync(grad_edge, 0, (size_t)b->nnz_total * sizeof(float), stream));
+    auto edge_step = [&](const float* ip) -> int {
+        if (!grad_edge) return GNODE_OK;
+        bwd_edge_kernel<<<pl.grid_row, ROW_THREADS, 0, stream>>>(a, ip, b->d_inst_e0, grad_edge);
+        GN_LAUNCH_CHECK();
+        return GNODE_OK;
+    };
 
     auto state = [&](int j) { return traj + (size_t)j * 3 * M * H; };
     // cotangent of grid point j, or null when its probabilities were not emitted (sparse dL/dprobs: the loss of the
@@ -1109,6 +1188,7 @@ extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int
             GN_LAUNCH_CHECK();
             bwd_gz_kernel<true><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
             GN_LAUNCH_CHECK();
+            if (const int rc2 = edge_step(a.Ipf)) return rc2;
             a.part = plin;
             return launch_vjp(a, pl.grid_tile3, wgrad, stream);
         }
@@ -1122,6 +1202,7 @@ extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int
         a.part = nullptr;
         bwd_gz_kernel<false><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
         GN_LAUNCH_CHECK();
+        if (const int rc2 = edge_step(a.Ip)) return rc2;
         a.part = plin;
         return launch_vjp(a, pl.grid_tile3, wgrad, stream);
     };

@@ -86,6 +86,7 @@ struct gnode_batch {
     int32_t n_tiles = 0;
     int64_t nnz_total = 0;
     GnInstance* d_inst = nullptr;    // [n_inst]
+    int64_t* d_inst_e0 = nullptr;    // [n_inst] first entry of each instance in the batch's edge vector (edge gradients)
     int32_t* d_tile_inst = nullptr;  // [n_tiles] instance that owns the first row of each tile
     int32_t* d_tile_order = nullptr; // [n_tiles] processing order: hub-heavy tiles first, then row-major
     int2* d_sched = nullptr;         // [n_tiles] by sequence number: {tile, first row of the look-ahead I' prefetch or -1}

@@ -163,6 +163,7 @@ extern "C" int gnode_batch_create(const gnode_graph_t* inst_graphs, int32_t n_in
         return GNODE_ERR_ARG;
     }
     std::vector<GnInstance> inst(n_inst);
+    std::vector<int64_t> inst_e0(n_inst);
     int64_t M = 0, nnz = 0;
     for (int32_t i = 0; i < n_inst; ++i) {
         const gnode_graph* g = inst_graphs[i];
@@ -170,6 +171,7 @@ extern "C" int gnode_batch_create(const gnode_graph_t* inst_graphs, int32_t n_in
         inst[i].rowptr = g->d_rowptr; inst[i].colidx = g->d_colidx;
         inst[i].rowptr_t = g->d_rowptr_t; inst[i].colidx_t = g->d_colidx_t;
         inst[i].row0 = (int32_t)M; inst[i].n = g->n;
+        inst_e0[i] = nnz;
         M += g->n; nnz += g->nnz;
         if (M > 0x7fffff00LL) { set_error("gnode_batch_create: %lld rows exceed the int32 row space", (long long)M); return GNODE_ERR_ARG; }
     }
@@ -261,6 +263,8 @@ extern "C" int gnode_batch_create(const gnode_graph_t* inst_graphs, int32_t n_in
     GN_CUDA(cudaMalloc(&b->d_tile_inst, sizeof(int32_t) * b->n_tiles));
     GN_CUDA(cudaMalloc(&b->d_tile_order, sizeof(int32_t) * b->n_tiles));
     GN_CUDA(cudaMemcpy(b->d_inst, inst.data(), sizeof(GnInstance) * n_inst, cudaMemcpyHostToDevice));
+    GN_CUDA(cudaMalloc(&b->d_inst_e0, sizeof(int64_t) * n_inst));
+    GN_CUDA(cudaMemcpy(b->d_inst_e0, inst_e0.data(), sizeof(int64_t) * n_inst, cudaMemcpyHostToDevice));
     GN_CUDA(cudaMemcpy(b->d_tile_inst, tile_inst.data(), sizeof(int32_t) * b->n_tiles, cudaMemcpyHostToDevice));
     GN_CUDA(cudaMemcpy(b->d_tile_order, order.data(), sizeof(int32_t) * b->n_tiles, cudaMemcpyHostToDevice));
     {   // schedule entries: tile + the row where the same tile of the NEXT instance starts (I' look-ahead prefetch)
@@ -387,6 +391,7 @@ extern "C" int gnode_batch_destroy(gnode_batch_t b) {
     for (auto& e : b->bwd_graphs) cudaGraphExecDestroy((cudaGraphExec_t)e.exec);
     if (b->capture_stream) cudaStreamDestroy((cudaStream_t)b->capture_stream);
     cudaFree(b->d_inst);
+    cudaFree(b->d_inst_e0);
     cudaFree(b->d_tile_inst);
     cudaFree(b->d_tile_order);
     cudaFree(b->d_sched);

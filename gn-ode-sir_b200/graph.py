@@ -14,7 +14,8 @@ from . import _lib
 
 
 class DeviceGraph:
-    """CSR pattern of one graph in HBM (gnode_graph_t)."""
+    """CSR pattern of one graph in HBM (gnode_graph_t). indptr / indices keep the host copy of what was uploaded: the
+    columns of every row in ascending order, the order of the device CSR and of the edge gradients."""
 
     def __init__(self, A):
         import scipy.sparse
@@ -23,7 +24,10 @@ class DeviceGraph:
             raise ValueError("adjacency must be square, got %r" % (A.shape,))
         self.n = int(A.shape[0])
         indptr = np.ascontiguousarray(A.indptr, dtype=np.int32)
-        indices = np.ascontiguousarray(A.indices, dtype=np.int32)
+        indices = np.asarray(A.indices[:indptr[-1]], dtype=np.int32)
+        rows = np.repeat(np.arange(self.n, dtype=np.int32), np.diff(indptr))
+        indices = np.ascontiguousarray(indices[np.lexsort((indices, rows))])      # per-row column sort
+        self.indptr, self.indices = indptr, indices
         self.nnz = int(indptr[-1])
         h = ctypes.c_void_p()
         L = _lib.lib()
@@ -35,6 +39,10 @@ class DeviceGraph:
         _lib.check(L.gnode_graph_info(h, ctypes.byref(n), ctypes.byref(nnz), ctypes.byref(md), ctypes.byref(sym)),
                    "gnode_graph_info")
         self.max_degree, self.symmetric = int(md.value), bool(sym.value)
+
+    def edges(self):
+        """(row, col) of every stored entry, int64, in the order of the edge gradients (rollout's edge_weight)."""
+        return np.repeat(np.arange(self.n, dtype=np.int64), np.diff(self.indptr)), self.indices.astype(np.int64)
 
     def __del__(self):
         try:
@@ -56,6 +64,9 @@ class DeviceBatch:
         self.handle = h
         self.M = int(_lib.lib().gnode_batch_rows(h))
         self.sizes = [g.n for g in self.graphs]
+        # edge vector of the batch (edge gradients): instance after instance, edge_offsets[i] = first entry of instance i
+        self.edge_offsets = np.concatenate(([0], np.cumsum([g.nnz for g in self.graphs]))).astype(np.int64)
+        self.nnz = int(self.edge_offsets[-1])
 
     def __del__(self):
         try:

@@ -94,7 +94,7 @@ def dt_array(integration_time):
 
 class _Rollout(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, batch, dt, grad_mode, want_grad, out_steps, *params):
+    def forward(ctx, x, batch, dt, grad_mode, want_grad, out_steps, edge_weight, *params):
         L = _lib.lib()
         M, T = batch.M, len(dt) + 1
         steps, steps_p, n_out = _steps_arg(out_steps, T)
@@ -130,8 +130,9 @@ class _Rollout(torch.autograd.Function):
         if need_grad:
             ctx.save_for_backward(x, traj, *ps)
             ctx.batch, ctx.dt, ctx.grad_mode, ctx.steps = batch, dt, grad_mode, steps
+            ctx.edge_shape = tuple(edge_weight.shape) if edge_weight is not None else None
             ctx.aux = aux if filled.value == 1 else None
-            ctx.wgrad = any(ctx.needs_input_grad[6:])       # False: input gradients only (no weight-gradient phase)
+            ctx.wgrad = any(ctx.needs_input_grad[7:])       # False: input gradients only (no weight-gradient phase)
         return probs
 
     @staticmethod
@@ -148,35 +149,56 @@ class _Rollout(torch.autograd.Function):
             grads = torch.empty(_lib.GRAD_COUNT, dtype=torch.float32, device=x.device) if ctx.wgrad else None
             # dL/dx: columns 0..4 written by the sweep, the others (graph marker, unused bg channels) carry no gradient
             grad_x = torch.zeros(tuple(x.shape), dtype=torch.float32, device=x.device) if ctx.needs_input_grad[0] else None
+            # dL/dw per stored adjacency entry (one float more than nnz keeps the pointer valid on edgeless batches)
+            grad_edge = torch.empty(batch.nnz + 1, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[6] else None
             ws_bytes = int(L.gnode_backward_workspace_bytes(batch.handle))
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
             pstruct = _params_struct(ps)
             mode = {"adjoint": _lib.GRAD_ADJOINT, "discrete": _lib.GRAD_DISCRETE}[ctx.grad_mode]
-            _lib.check(L.gnode_rollout_backward_input(batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T,
+            _lib.check(L.gnode_rollout_backward_edges(batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T,
                                                       dt.ctypes.data_as(_lib.c_float_p), _ptr(traj),
                                                       _ptr(ctx.aux) if ctx.aux is not None else None, _ptr(grad_probs),
                                                       steps_p, len(steps) if steps is not None else 0, mode,
                                                       _ptr(grads) if grads is not None else None,
                                                       _ptr(grad_x) if grad_x is not None else None,
                                                       grad_x.stride(0) if grad_x is not None else 0,
+                                                      _ptr(grad_edge) if grad_edge is not None else None,
                                                       _ptr(ws), ws_bytes, _stream(x.device)),
-                       "gnode_rollout_backward_input")
+                       "gnode_rollout_backward_edges")
         out, off = [], 0
         for i, (k, shape) in enumerate(_lib.GRAD_LAYOUT):
             n = int(np.prod(shape))
-            out.append(grads[off:off + n].view(shape) if ctx.needs_input_grad[6 + i] else None)
+            out.append(grads[off:off + n].view(shape) if ctx.needs_input_grad[7 + i] else None)
             off += n
-        return (grad_x, None, None, None, None, None, *out)
+        ge = grad_edge[:batch.nnz].view(ctx.edge_shape) if grad_edge is not None else None
+        return (grad_x, None, None, None, None, None, ge, *out)
 
 
-def rollout(x, batch, dt, params, grad_mode="adjoint", out_steps=None):
+def _check_edge_weight(edge_weight, batch):
+    """edge_weight: the unit weights of the batch's stored adjacency entries, there to receive dL/dw. The forward runs
+    the binary adjacency, so every weight must be 1 (one device-wide check, on this opt-in path only)."""
+    _check_cuda_f32(edge_weight, "edge_weight")
+    if edge_weight.numel() != batch.nnz:
+        raise ValueError("edge_weight must hold one value per stored adjacency entry of the batch (%d), got %d"
+                         % (batch.nnz, edge_weight.numel()))
+    if not bool(torch.all(edge_weight.detach() == 1)):
+        raise ValueError("edge_weight must be all ones: the rollout runs the binary adjacency and edge_weight only "
+                         "receives dL/dw; to remove an edge, build a graph without it")
+
+
+def rollout(x, batch, dt, params, grad_mode="adjoint", out_steps=None, edge_weight=None):
     """x [M, >=5] -> probabilities [T, M, 3] (or [len(out_steps), M, 3]: only those grid points are decoded and
     stored); params in PARAM_ORDER (state_dict names). Differentiable with respect to the parameters and to x (columns
-    S0, I0, R0, beta, gamma; the other columns get zero gradients)."""
+    S0, I0, R0, beta, gamma; the other columns get zero gradients). edge_weight: an all-ones float32 CUDA tensor with
+    batch.nnz elements (instance after instance, each in DeviceGraph.edges() order); when it requires grad it receives
+    dL/dw of every stored adjacency entry, the gradient of the weighted neighbour sum at w = 1."""
     if grad_mode not in ("adjoint", "discrete"):
         raise ValueError("grad_mode must be 'adjoint' or 'discrete'")
-    want_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
-    return _Rollout.apply(x, batch, dt, grad_mode, want_grad, out_steps, *params)
+    if edge_weight is not None:
+        _check_edge_weight(edge_weight, batch)
+    want_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params) or
+                                             (edge_weight is not None and edge_weight.requires_grad))
+    return _Rollout.apply(x, batch, dt, grad_mode, want_grad, out_steps, edge_weight, *params)
 
 
 class TrialSet:
@@ -270,14 +292,17 @@ class _ExpandTrials(torch.autograd.Function):
 
 
 def rollout_trials(batch, trials, dt, params, grad_mode="adjoint", out_steps=None, probs_out=None, workspace=None,
-                   beta=None, gamma=None):
+                   beta=None, gamma=None, edge_weight=None):
     """Rollout straight from compact trial descriptors. Without gradients: ONE C-ABI call (expansion into the
     workspace + rollout), optionally into caller-owned `probs_out` / `workspace` buffers (streaming loops reuse them).
     With gradients: the compact x is kept for the reverse sweep. `beta` / `gamma`: the tensors the set was made from;
     when one of them requires grad, it receives dL/dbeta[i] (dL/dgamma[i]) per instance. Seed sets are discrete and
-    have no gradient."""
+    have no gradient. `edge_weight`: as for rollout() ([B, nnz] for B trials of one graph)."""
+    if edge_weight is not None:
+        _check_edge_weight(edge_weight, batch)
     want_x = torch.is_grad_enabled() and any(torch.is_tensor(v) and v.requires_grad for v in (beta, gamma))
-    want_grad = want_x or (torch.is_grad_enabled() and any(p.requires_grad for p in params))
+    want_grad = want_x or (torch.is_grad_enabled() and (any(p.requires_grad for p in params) or
+                                                        (edge_weight is not None and edge_weight.requires_grad)))
     if want_grad:
         if want_x:
             bt = beta if torch.is_tensor(beta) else trials.beta
@@ -287,7 +312,7 @@ def rollout_trials(batch, trials, dt, params, grad_mode="adjoint", out_steps=Non
             x = _ExpandTrials.apply(bt, gt, batch, trials)
         else:
             x = expand_trials(batch, trials)
-        return rollout(x, batch, dt, params, grad_mode, out_steps)
+        return rollout(x, batch, dt, params, grad_mode, out_steps, edge_weight)
     L = _lib.lib()
     if trials.n_inst != len(batch.sizes):
         raise ValueError("%d trial descriptors for a batch of %d instances" % (trials.n_inst, len(batch.sizes)))

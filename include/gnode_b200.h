@@ -255,6 +255,24 @@ int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int64_t ldx, c
                                  const int32_t* out_steps, int32_t n_out, int32_t grad_mode, float* grads_out,
                                  float* grad_x, int64_t ldgx, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- edge gradients: dL/dw per stored adjacency entry ------------------------------
+ * The forward is the reference's binary adjacency; the gradient is that of the weighted neighbour sum
+ * AI[r] = sum_c w_rc I'[c], taken at w = 1 (what contact reduction, edge removal and structural attribution rank by).
+ * Per reverse step, at the same state and dt as the parameter VJP (ADJOINT: y_i with a_i; DISCRETE: exact
+ * back-propagation of the Euler loop), with gAI = beta (aI - aS) S':
+ *   dL/dw_rc += dt * sum_h gAI[r,h] I'[c,h]          for every stored entry (r, c) of A
+ * Row sums tie it to grad_x: sum over row r's entries of dL/dw_rc = beta[r] * dL/dbeta[r].
+ *   grad_edge  [nnz_total] or NULL: overwritten with dL/dw. Layout: instance after instance (in batch order), inside an
+ *              instance the graph's CSR order after gnode_graph_create's per-row column sort.
+ * Arguments otherwise as gnode_rollout_backward_input (which is this call with grad_edge == NULL, bit for bit); at least
+ * one of grads_out / grad_x / grad_edge non-NULL. Same workspace. One more row kernel per reverse step when grad_edge is
+ * non-NULL; one lane per edge adds its fixed-order dot product (no atomics): bitwise reproducible. */
+int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p, int32_t T,
+                                 const float* dt_host, const float* traj, const float* aux, const float* grad_probs,
+                                 const int32_t* out_steps, int32_t n_out, int32_t grad_mode, float* grads_out,
+                                 float* grad_x, int64_t ldgx, float* grad_edge, void* workspace, size_t workspace_bytes,
+                                 void* stream);
+
 /* Per-instance sums of grad_x columns 3 and 4 (instance i = rows [row0_i, row0_i + n_i)), in a fixed order:
  * the gradient of compact trial descriptors' beta[i], gamma[i] (N4). grad_beta, grad_gamma: DEVICE float[n_inst]. */
 int gnode_trials_grad(gnode_batch_t b, const float* grad_x, int64_t ldgx, float* grad_beta, float* grad_gamma,
