@@ -84,6 +84,14 @@ SIGNATURES = {
     "gnode_rollout_backward_edges": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(GnodeParams), c_int32,
                                              c_float_p, c_void_p, c_void_p, c_void_p, c_int32_p, c_int32, c_int32,
                                              c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gnode_rollout_forward_weighted": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(GnodeParams), c_int32,
+                                               c_float_p, c_int32_p, c_int32, c_void_p, c_void_p, c_int32_p, c_void_p,
+                                               c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gnode_backward_weighted_workspace_bytes": (c_size_t, [c_void_p]),
+    "gnode_rollout_backward_weighted": (c_int, [c_void_p, c_void_p, c_int64, ctypes.POINTER(GnodeParams), c_int32,
+                                                c_float_p, c_void_p, c_void_p, c_void_p, c_int32_p, c_int32, c_int32,
+                                                c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_size_t,
+                                                c_void_p]),
     "gnode_trials_grad": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "gnode_mc_sir_workspace_bytes": (c_size_t, [c_void_p, c_int32]),
     "gnode_mc_sir": (c_int, [c_void_p, c_void_p, c_int32, ctypes.c_float, ctypes.c_float, c_int32, c_int32,

@@ -21,6 +21,8 @@
 //   K2 bwd_row_kernel       : AI = A I' ; a += D(y_j,gP_j) (adjoint mode) ; gAI   -> AI, G, a
 //                             (discrete mode adds D in a separate row pass after K3)
 //   K3a bwd_gz_kernel      : A^T gAI, gz* (in place over Sp / AI)
+// Weighted sweeps (gnode_rollout_backward_weighted) gather sum_c w_rc I'[c] in K2 and sum_c w_cr gAI[c] in K3a (the
+// weights in transpose order, permuted once per sweep by permute_weights_kernel); K3e's formula holds at any w.
 //   K3e bwd_edge_kernel    : dL/dw_rc += dt * gAI[r] . I'[c] per stored entry of A (only when edge gradients are asked)
 //   K3 bwd_vjp_kernel       : per-CTA vW / vb (FFMA), v = gz W into a (tcgen05)
 // Parameter-gradient partial sums live in per-CTA slots (no atomics: bitwise reproducible) and are
@@ -59,6 +61,9 @@ struct BwdArgs {
     float dt;
     int only_dec;                  // 1: only a += D(y, gP)
     gnode_params_t p;
+    // weighted neighbour sum (the W instantiations): weight of forward entry e of instance i = ew[inst_e0[i] + e], of
+    // transpose entry k = ewT[inst_e0[i] + k] (ew permuted by the graph's transpose map)
+    const float* ew; const float* ewT; const int64_t* inst_e0;
 };
 
 // ---------------------------------------------------------------- K1
@@ -235,6 +240,7 @@ __device__ __forceinline__ void decoder_backward_row(const float4 (&c)[3], const
 // ---------------------------------------------------------------- K2
 // (3 CTAs per SM at 80 registers; 2 CTAs at 128 registers without spills, and issuing the own-row loads before the
 // gather, measured no better: profiles/r1e_ab_backward.log)
+template <bool W>
 __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_row_kernel(const BwdArgs a) {
     __shared__ float W3s[4 * H];
     __shared__ float small[12];
@@ -266,6 +272,7 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_row_kernel(const BwdArgs a
         float be = 0.f;
         int row0 = 0, e0 = 0, deg = 0;
         const int32_t* ci = nullptr;
+        const float* wp = nullptr;
         if (!a.only_dec) {
             if (valid) {
                 int inst = a.bv.tile_inst[g / TILE];                 // owner of the tile's first row, then walk forward
@@ -276,8 +283,9 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_row_kernel(const BwdArgs a
                 e0 = I.rowptr[n];
                 deg = I.rowptr[n + 1] - e0;
                 be = a.x[(size_t)g * a.ldx + 3];
+                if (W) wp = a.ew + a.inst_e0[inst];
             }
-            AI = gather_row(a.Ip, ci, e0, deg, row0, l, lane);
+            AI = gather_row<W>(a.Ip, ci, e0, deg, row0, l, lane, wp);
         }
         // Grid points without a cotangent (sparse dL/dprobs: only the rows int(i/deltaT) enter the loss) have D = 0:
         // no decoder backward, the state planes are not read and the adjoint is not rewritten
@@ -404,7 +412,8 @@ __global__ void __launch_bounds__(ROW_THREADS, 2) bwd_dec_kernel(const BwdArgs a
 //   gzI = (A^T gAI + gamma (aR - aI)) I'(1-I')      gzS = beta (aI - aS) AI S'(1-S')
 // written IN PLACE over the row's own S' (Sp <- gzS) and AI (AI <- gzI): both are read only by this row's threads.
 // Separate from the tile kernel so that this latency-bound gather runs at row-kernel occupancy.
-template <bool AUX>       // AUX: gzS was written by bwd_transform_g_kernel; I' comes from the forward's auxiliary storage
+// AUX: gzS was written by bwd_transform_g_kernel; I' comes from the forward's auxiliary storage. W: A^T of the weighted sum
+template <bool AUX, bool W>
 __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_gz_kernel(const BwdArgs a) {
     const int tid = threadIdx.x, lane = tid & 31, l = tid & 15, hw = tid >> 4;
     const int M = a.bv.M;
@@ -417,6 +426,7 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_gz_kernel(const BwdArgs a)
         const size_t off = (size_t)(valid ? g : 0) * H + 4 * l;
         int row0 = 0, e0 = 0, deg = 0;
         const int32_t* ci = nullptr;
+        const float* wp = nullptr;
         float be = 0.f, ga = 0.f;
         float4 aS, aI, aR, sp, ip, ai;
         if (valid) {
@@ -437,8 +447,9 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_gz_kernel(const BwdArgs a)
             deg = I.rowptr_t[n + 1] - e0;
             be = a.x[(size_t)g * a.ldx + 3];
             ga = a.x[(size_t)g * a.ldx + 4];
+            if (W) wp = a.ewT + a.inst_e0[inst];
         }
-        const float4 gsum = gather_row(a.G, ci, e0, deg, row0, l, lane);
+        const float4 gsum = gather_row<W>(a.G, ci, e0, deg, row0, l, lane, wp);
         if (valid) {
             float4 gzs, gzi;
 #define GN_GZ(c)                                                               \
@@ -529,6 +540,22 @@ __global__ void __launch_bounds__(ROW_THREADS, 3) bwd_edge_kernel(const BwdArgs 
             }
             if (eb + l < deg) out[eb + l] += a.dt * res;
         }
+    }
+}
+
+// ---------------------------------------------------------------- weights in transpose order (weighted sweeps)
+// wT[inst_e0[i] + k] = w[inst_e0[i] + tmap_i[k]]: transpose entry k of instance i is forward entry tmap_i[k] of its graph
+__global__ void __launch_bounds__(256) permute_weights_kernel(const float* __restrict__ w, const int32_t* const* __restrict__ tmaps,
+                                                              const int64_t* __restrict__ inst_e0, int n_inst, int64_t nnz,
+                                                              float* __restrict__ wT) {
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < nnz; k += (int64_t)gridDim.x * blockDim.x) {
+        int lo = 0, hi = n_inst - 1;                      // last instance with inst_e0 <= k (edgeless ones share their e0)
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (inst_e0[mid] <= k) lo = mid; else hi = mid - 1;
+        }
+        const int64_t e0 = inst_e0[lo];
+        wT[k] = w[e0 + tmaps[lo][k - e0]];
     }
 }
 
@@ -1058,11 +1085,26 @@ extern "C" int gnode_rollout_backward_input(gnode_batch_t b, const float* x, int
                                         grads_out, grad_x, ldgx, nullptr, workspace, workspace_bytes, stream_);
 }
 
+extern "C" size_t gnode_backward_weighted_workspace_bytes(gnode_batch_t b) {
+    if (!b) return 0;
+    return plan_backward(b).total + align_up((size_t)std::max<int64_t>(b->nnz_total, 1) * sizeof(float), 256);
+}
+
 extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p,
                                             int32_t T, const float* dt_host, const float* traj, const float* aux,
                                             const float* grad_probs, const int32_t* out_steps, int32_t n_out,
                                             int32_t grad_mode, float* grads_out, float* grad_x, int64_t ldgx,
                                             float* grad_edge, void* workspace, size_t workspace_bytes, void* stream_) {
+    return gnode_rollout_backward_weighted(b, x, ldx, p, T, dt_host, traj, aux, grad_probs, out_steps, n_out, grad_mode,
+                                           grads_out, grad_x, ldgx, grad_edge, nullptr, workspace, workspace_bytes, stream_);
+}
+
+extern "C" int gnode_rollout_backward_weighted(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p,
+                                               int32_t T, const float* dt_host, const float* traj, const float* aux,
+                                               const float* grad_probs, const int32_t* out_steps, int32_t n_out,
+                                               int32_t grad_mode, float* grads_out, float* grad_x, int64_t ldgx,
+                                               float* grad_edge, const float* edge_w, void* workspace,
+                                               size_t workspace_bytes, void* stream_) {
     if (!b || !x || !p || !traj || !grad_probs || (!grads_out && !grad_x && !grad_edge) || (grad_x && ldgx < 5) ||
         !workspace || T < 1 || ldx < 5 || (T > 1 && !dt_host) ||
         (grad_mode != GNODE_GRAD_ADJOINT && grad_mode != GNODE_GRAD_DISCRETE)) {
@@ -1077,10 +1119,12 @@ extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int
     if (rc) return rc;
     if ((rc = check_current_device(b, "gnode_rollout_backward"))) return rc;
     const BwdPlan pl = plan_backward(b);
-    if (workspace_bytes < pl.total) {
-        set_error("gnode_rollout_backward: workspace too small (%zu < %zu)", workspace_bytes, pl.total);
+    const size_t ws_need = edge_w ? gnode_backward_weighted_workspace_bytes(b) : pl.total;
+    if (workspace_bytes < ws_need) {
+        set_error("gnode_rollout_backward: workspace too small (%zu < %zu)", workspace_bytes, ws_need);
         return GNODE_ERR_ARG;
     }
+    if (edge_w && (rc = ensure_transpose_maps(b))) return rc;
     cudaStream_t stream = (cudaStream_t)stream_;
     static bool configured[64] = {false};
     if (!configured[b->device & 63]) {
@@ -1109,8 +1153,9 @@ extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int
                 if (key == 0) key = 1469598103934665603ull;
                 for (size_t i = 0; i < n; ++i) { key ^= c[i]; key *= 1099511628211ull; }
             };
-            // (grads_out == NULL, i.e. no parameter gradient, grad_x == NULL and grad_edge == NULL are part of the pointers)
-            const void* ptrs[] = {x, traj, aux, grad_probs, grads_out, workspace, stream_, grad_x, grad_edge};
+            // (grads_out == NULL, i.e. no parameter gradient, grad_x == NULL, grad_edge == NULL and edge_w == NULL are part of
+            // the pointers; the weights' values are read inside the graph, so new values written in place are honoured)
+            const void* ptrs[] = {x, traj, aux, grad_probs, grads_out, workspace, stream_, grad_x, grad_edge, edge_w};
             mix(ptrs, sizeof(ptrs)); mix(p, sizeof(*p)); mix(&ldx, sizeof(ldx)); mix(&T, sizeof(T));
             mix(&ldgx, sizeof(ldgx));
             mix(&grad_mode, sizeof(grad_mode)); mix(dt_host, sizeof(float) * (size_t)(T > 1 ? T - 1 : 0));
@@ -1149,6 +1194,13 @@ extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int
     float* pdec = (float*)(ws + pl.off_pdec);
     float* plin = (float*)(ws + pl.off_plin);
     float* penc = (float*)(ws + pl.off_penc);
+    a.ew = edge_w; a.ewT = edge_w ? (float*)(ws + pl.total) : nullptr; a.inst_e0 = b->d_inst_e0;
+    if (edge_w && b->nnz_total > 0) {            // the weights in transpose order, for the A^T gather of every step
+        const int grid = (int)std::min<int64_t>((b->nnz_total + 255) / 256, (int64_t)b->sm_count * 8);
+        permute_weights_kernel<<<grid, 256, 0, stream>>>(edge_w, b->d_inst_tmap, b->d_inst_e0, b->n_inst, b->nnz_total,
+                                                         (float*)(ws + pl.total));
+        GN_LAUNCH_CHECK();
+    }
     // adjoint and partial-sum slots start at zero
     GN_CUDA(cudaMemsetAsync(ws + pl.off_a, 0, 3 * M * H * sizeof(float), stream));
     GN_CUDA(cudaMemsetAsync(ws + pl.off_pdec, 0, pl.off_penc - pl.off_pdec, stream));
@@ -1186,7 +1238,8 @@ extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int
             a.Ipf = aux + (size_t)j * 2 * aux_plane; a.AIf = a.Ipf + aux_plane;
             bwd_transform_g_kernel<<<pl.grid_tile1, NTHREADS, K1_SM_TOTAL, stream>>>(a);
             GN_LAUNCH_CHECK();
-            bwd_gz_kernel<true><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
+            if (edge_w) bwd_gz_kernel<true, true><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
+            else bwd_gz_kernel<true, false><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
             GN_LAUNCH_CHECK();
             if (const int rc2 = edge_step(a.Ipf)) return rc2;
             a.part = plin;
@@ -1197,10 +1250,12 @@ extern "C" int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int
         bwd_transform_kernel<<<pl.grid_tile1, NTHREADS, K1_SM_TOTAL, stream>>>(a);
         GN_LAUNCH_CHECK();
         a.part = pdec;
-        bwd_row_kernel<<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
+        if (edge_w) bwd_row_kernel<true><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
+        else bwd_row_kernel<false><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
         GN_LAUNCH_CHECK();
         a.part = nullptr;
-        bwd_gz_kernel<false><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
+        if (edge_w) bwd_gz_kernel<false, true><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
+        else bwd_gz_kernel<false, false><<<pl.grid_row, ROW_THREADS, 0, stream>>>(a);
         GN_LAUNCH_CHECK();
         if (const int rc2 = edge_step(a.Ip)) return rc2;
         a.part = plin;

@@ -54,6 +54,9 @@ struct OutSel {
 int make_out_sel(int T, const int32_t* out_steps, int32_t n_out, OutSel* o, const char* what);
 // GNODE_ERR_ARG unless the handle's device is the calling thread's current device
 int check_current_device(const gnode_batch* b, const char* what);
+// weighted reverse sweep: uploads (once) the transpose -> forward entry maps of the batch's graphs and the per-instance
+// table of them (b->d_inst_tmap); a blocking call, made before any capture starts
+int ensure_transpose_maps(gnode_batch* b);
 }  // namespace gnode
 
 // One graph: CSR pattern (and its transpose) resident in HBM.
@@ -67,6 +70,10 @@ struct gnode_graph {
     int32_t* d_rowptr_t = nullptr;  // transpose (aliases the above when symmetric)
     int32_t* d_colidx_t = nullptr;
     std::vector<int32_t> h_rowptr;  // host copy (tile cost model at batch creation)
+    // transpose entry k (of the counting sort below) is forward entry h_tmap[k]: the order a weight vector takes for the
+    // A^T gather of the weighted reverse sweep (symmetric graphs too: the pattern is shared, the weights need not be)
+    std::vector<int32_t> h_tmap;
+    int32_t* d_tmap = nullptr;      // uploaded on first weighted use
     int device = 0;
 };
 
@@ -99,6 +106,8 @@ struct gnode_batch {
     struct BwdGraph { uint64_t key; void* exec; int64_t kernels; };
     std::vector<BwdGraph> bwd_graphs;
     void* capture_stream = nullptr;      // cudaStream_t used only to capture those graphs
+    std::vector<gnode_graph*> graphs;    // the instances' graphs (the caller keeps them alive while the batch lives)
+    const int32_t** d_inst_tmap = nullptr;   // [n_inst] graph's transpose map per instance (weighted sweeps), or null
 };
 
 // Kernel-side view of a batch.
@@ -154,6 +163,12 @@ __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 r; asm(
 __device__ __forceinline__ void add4(float4& acc, const float4& v) {
     unpack2(add2(pack2(acc.x, acc.y), pack2(v.x, v.y)), acc.x, acc.y);
     unpack2(add2(pack2(acc.z, acc.w), pack2(v.z, v.w)), acc.z, acc.w);
+}
+
+// w * v component by component, each product rounded on its own: scalar mul.rn is never contracted with the add that
+// follows (the weighted neighbour sums add fl(w v) in the same order as the binary ones add v; w = 1 gives their bits)
+__device__ __forceinline__ float4 mul4(float w, const float4& v) {
+    return make_float4(__fmul_rn(w, v.x), __fmul_rn(w, v.y), __fmul_rn(w, v.z), __fmul_rn(w, v.w));
 }
 
 __device__ __forceinline__ float4 lds4(const unsigned char* base, int off) {

@@ -79,6 +79,9 @@ struct StepArgs {
     // step_stream_kernel: the S_k tile arrives by TMA tensor loads (same box / swizzle = the UMMA operand layout)
     alignas(64) CUtensorMap tm_s_in;     // [M rows][64] fp32 over the S plane of y_in (one launch per step)
     alignas(64) CUtensorMap tm_sp[2];    // persistent rollout: over the S planes of st[0] / st[1], or [0] over the whole trajectory
+    // weighted neighbour sum (step_stream_kernel, OPT bit 8): weight of entry e of instance i = edge_w[inst_e0[i] + e]
+    const float* edge_w;
+    const int64_t* inst_e0;
 };
 
 // output slot of grid point k (-1: its probabilities are not emitted)
@@ -579,8 +582,10 @@ __device__ __forceinline__ float4 gather_smem_nb(const float* __restrict__ lane_
 
 // K neighbour rows, no predication: slots past the row's degree read the all-zero row `zrow` of the I' buffer
 // (adding +0 is exact), so the loads need neither a zero-initialised destination nor a predicate.
-template <int K>
-__device__ __forceinline__ void gather_exact(float4& acc, const float* __restrict__ lane_base, const int* cp, int j0, int deg, int zrow, uint64_t pol) {
+// W: weighted, acc += fl(wp[j] v_j); the weights are read after the loads are issued (pad slots: weight 0, row 0)
+template <int K, bool W = false>
+__device__ __forceinline__ void gather_exact(float4& acc, const float* __restrict__ lane_base, const int* cp, int j0, int deg, int zrow, uint64_t pol,
+                                             const float* wp = nullptr) {
     float4 v[K];
 #pragma unroll
     for (int k = 0; k < K; ++k) {
@@ -588,7 +593,10 @@ __device__ __forceinline__ void gather_exact(float4& acc, const float* __restric
         v[k] = ldg4_hint(lane_base + (size_t)(unsigned)c * H, pol);
     }
 #pragma unroll
-    for (int k = 0; k < K; ++k) add4(acc, v[k]);
+    for (int k = 0; k < K; ++k) {
+        if (W) v[k] = mul4((j0 + k < deg) ? wp[j0 + k] : 0.f, v[k]);
+        add4(acc, v[k]);
+    }
 }
 
 // Warp-uniform neighbour sum specialised by the pair's larger degree (1..12 in one round trip, longer rows in
@@ -1312,6 +1320,17 @@ static bool use_dual() { return (current_variant() & VAR_TC) && step_kernel_choi
 template <int MODE>
 static int launch_step(const gnode_batch* b, const StepArgs& a, cudaStream_t stream) {
     const int var = current_variant();
+    if (MODE == MODE_STEP && a.edge_w) {                       // weighted neighbour sum: the default step kernel only
+        if (!use_dual() || step_kernel_choice() != 5 || a.use_tma != 2) {
+            set_error("gnode_rollout_forward_weighted: the weighted neighbour sum runs only on step kernel 5 with TMA-fed "
+                      "operands (tensor-core variant, tensor maps available); current step kernel %d, variant %d",
+                      step_kernel_choice(), var);
+            return GNODE_ERR_UNSUPPORTED;
+        }
+        const bool fast = (var & VAR_FASTSIG) != 0, rf = a.hid_r != nullptr;
+        return fast ? (rf ? launch_step_stream<true, true, 321>(b, a, stream) : launch_step_stream<true, false, 321>(b, a, stream))
+                    : (rf ? launch_step_stream<false, true, 321>(b, a, stream) : launch_step_stream<false, false, 321>(b, a, stream));
+    }
     if (MODE == MODE_STEP && use_dual()) {
         if (step_kernel_choice() >= 5 && a.use_tma == 2) {      // TMA-fed S stream (6: without the deferred store wait)
             const bool fast = (var & VAR_FASTSIG) != 0, rf = a.hid_r != nullptr;
@@ -1533,8 +1552,14 @@ static int launch_encode_trials(const gnode_batch* b, const StepArgs& a, const T
 static int rollout_forward_impl(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p, int32_t T,
                                 const float* dt_host, const OutSel& sel, float* traj, float* aux, int32_t* aux_filled,
                                 float* probs, void* workspace, size_t workspace_bytes, cudaStream_t stream,
-                                const TrialDesc* td = nullptr) {
+                                const TrialDesc* td = nullptr, const float* edge_w = nullptr) {
     if (aux_filled) *aux_filled = 0;
+    if (edge_w && (td || !use_dual() || step_kernel_choice() != 5 || tensor_map_encoder() == nullptr)) {
+        set_error("gnode_rollout_forward_weighted: the weighted neighbour sum runs only on step kernel 5 (current: %d) with "
+                  "the tensor-core variant (current: %d) and tensor maps (%s)", step_kernel_choice(), current_variant(),
+                  tensor_map_encoder() ? "available" : "not available on this driver");
+        return GNODE_ERR_UNSUPPORTED;
+    }
     if (workspace_bytes < gnode_rollout_workspace_bytes(b, traj != nullptr)) {
         set_error("gnode_rollout_forward: workspace too small (%zu < %zu)", workspace_bytes,
                   gnode_rollout_workspace_bytes(b, traj != nullptr));
@@ -1590,6 +1615,7 @@ static int rollout_forward_impl(gnode_batch_t b, const float* x, int64_t ldx, co
     a.out_slot = nullptr; a.out_start = sel.start; a.out_stride = sel.stride; a.n_out = sel.n_out;
     a.dbg = debug_flags();
     a.relay_off = g_hub_relay ? 0 : 1;
+    a.edge_w = edge_w; a.inst_e0 = b->d_inst_e0;
     a.tbuf = nullptr;
     if (a.dbg & 128) {
         if (!g_tbuf) { GN_CUDA(cudaMalloc(&g_tbuf, 64)); GN_CUDA(cudaMemset(g_tbuf, 0, 64)); }
@@ -1775,6 +1801,21 @@ extern "C" int gnode_rollout_forward_aux(gnode_batch_t b, const float* x, int64_
     int rc = make_out_sel(T, out_steps, n_out, &sel, "gnode_rollout_forward_aux");
     if (rc) return rc;
     return rollout_forward_impl(b, x, ldx, p, T, dt_host, sel, traj, aux, aux_filled, probs, workspace, workspace_bytes, (cudaStream_t)stream_);
+}
+
+extern "C" int gnode_rollout_forward_weighted(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p,
+                                              int32_t T, const float* dt_host, const int32_t* out_steps, int32_t n_out,
+                                              float* traj, float* aux, int32_t* aux_filled, float* probs,
+                                              const float* edge_w, void* workspace, size_t workspace_bytes, void* stream_) {
+    if (!b || !x || !p || !probs || !workspace || T < 1 || ldx < 5 || (T > 1 && !dt_host) || (aux && (!traj || !aux_filled))) {
+        set_error("gnode_rollout_forward_weighted: bad arguments (T=%d ldx=%lld)", T, (long long)ldx);
+        return GNODE_ERR_ARG;
+    }
+    OutSel sel;
+    int rc = make_out_sel(T, out_steps, n_out, &sel, "gnode_rollout_forward_weighted");
+    if (rc) return rc;
+    return rollout_forward_impl(b, x, ldx, p, T, dt_host, sel, traj, aux, aux_filled, probs, workspace, workspace_bytes,
+                                (cudaStream_t)stream_, nullptr, edge_w);
 }
 
 extern "C" int gnode_expand_trials(gnode_batch_t b, const int32_t* seeds, const int32_t* seed_ptr, const float* beta,

@@ -92,13 +92,13 @@ extern "C" int gnode_graph_create(int32_t n, int64_t nnz, const int32_t* rowptr,
         maxdeg = std::max(maxdeg, rowptr[r + 1] - rowptr[r]);
     }
     // transpose pattern by counting sort (rows ascending -> columns of A^T ascending)
-    std::vector<int32_t> rpt(n + 1, 0), cit(nnz);
+    std::vector<int32_t> rpt(n + 1, 0), cit(nnz), tmap(nnz);
     for (int64_t e = 0; e < nnz; ++e) rpt[ci[e] + 1]++;
     for (int32_t r = 0; r < n; ++r) rpt[r + 1] += rpt[r];
     {
         std::vector<int32_t> fill(rpt.begin(), rpt.end() - 1);
         for (int32_t r = 0; r < n; ++r)
-            for (int32_t e = rowptr[r]; e < rowptr[r + 1]; ++e) cit[fill[ci[e]]++] = r;
+            for (int32_t e = rowptr[r]; e < rowptr[r + 1]; ++e) { tmap[fill[ci[e]]] = e; cit[fill[ci[e]]++] = r; }
     }
     const bool sym = (memcmp(rpt.data(), rowptr, sizeof(int32_t) * (n + 1)) == 0) &&
                      (nnz == 0 || memcmp(cit.data(), ci.data(), sizeof(int32_t) * nnz) == 0);
@@ -106,6 +106,7 @@ extern "C" int gnode_graph_create(int32_t n, int64_t nnz, const int32_t* rowptr,
     gnode_graph* g = new gnode_graph();
     g->n = n; g->nnz = nnz; g->max_degree = maxdeg; g->symmetric = sym ? 1 : 0;
     g->h_rowptr.assign(rowptr, rowptr + n + 1);
+    g->h_tmap.swap(tmap);
     // device side: any CUDA failure frees what was allocated so far together with the handle
     auto upload = [&]() -> int {
     GN_CUDA(cudaGetDevice(&g->device));
@@ -144,6 +145,7 @@ extern "C" int gnode_graph_destroy(gnode_graph_t g) {
     }
     cudaFree(g->d_rowptr);
     cudaFree(g->d_colidx);
+    cudaFree(g->d_tmap);
     delete g;
     return GNODE_OK;
 }
@@ -177,6 +179,7 @@ extern "C" int gnode_batch_create(const gnode_graph_t* inst_graphs, int32_t n_in
     }
     gnode_batch* b = new gnode_batch();
     b->M = M; b->n_inst = n_inst; b->nnz_total = nnz;
+    b->graphs.assign(inst_graphs, inst_graphs + n_inst);
     b->n_tiles = (int32_t)((M + TILE - 1) / TILE);
     std::vector<int32_t> tile_inst(b->n_tiles);
     std::vector<int64_t> tile_cost(b->n_tiles, 0);
@@ -392,6 +395,7 @@ extern "C" int gnode_batch_destroy(gnode_batch_t b) {
     if (b->capture_stream) cudaStreamDestroy((cudaStream_t)b->capture_stream);
     cudaFree(b->d_inst);
     cudaFree(b->d_inst_e0);
+    cudaFree(b->d_inst_tmap);
     cudaFree(b->d_tile_inst);
     cudaFree(b->d_tile_order);
     cudaFree(b->d_sched);
@@ -403,6 +407,32 @@ extern "C" int gnode_batch_destroy(gnode_batch_t b) {
 }
 
 extern "C" int64_t gnode_batch_rows(gnode_batch_t b) { return b ? b->M : -1; }
+
+namespace gnode {
+int ensure_transpose_maps(gnode_batch* b) {
+    if (b->d_inst_tmap) return GNODE_OK;
+    std::vector<const int32_t*> maps(b->n_inst);
+    for (int32_t i = 0; i < b->n_inst; ++i) {
+        gnode_graph* g = b->graphs[i];
+        if (!g->d_tmap) {
+            int32_t* d = nullptr;
+            GN_CUDA(cudaMalloc(&d, sizeof(int32_t) * (size_t)std::max<int64_t>(g->nnz, 1)));
+            if (g->nnz) {
+                const cudaError_t e = cudaMemcpy(d, g->h_tmap.data(), sizeof(int32_t) * g->nnz, cudaMemcpyHostToDevice);
+                if (e != cudaSuccess) { cudaFree(d); GN_CUDA(e); }
+            }
+            g->d_tmap = d;
+        }
+        maps[i] = g->d_tmap;
+    }
+    const int32_t** d = nullptr;
+    GN_CUDA(cudaMalloc(&d, sizeof(const int32_t*) * b->n_inst));
+    const cudaError_t e = cudaMemcpy(d, maps.data(), sizeof(const int32_t*) * b->n_inst, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { cudaFree(d); GN_CUDA(e); }
+    b->d_inst_tmap = d;
+    return GNODE_OK;
+}
+}  // namespace gnode
 
 extern "C" int gnode_aggregate(gnode_batch_t b, const float* in, float* out, int transpose, void* stream) {
     if (!b || !in || !out) { set_error("gnode_aggregate: null argument"); return GNODE_ERR_ARG; }

@@ -36,12 +36,13 @@ struct StreamCfg {
     static constexpr int TR = 128;                         // tile rows = UMMA M
     static constexpr int RSTEP = PT / 16;                  // rows per pass of the row-per-half-warp loops (32)
     static constexpr int PASS = RSTEP * 128;               // byte offset between the passes' rows in an operand tile
-    static constexpr int CAP = 3 * PT;                     // colidx entries staged per tile
+    static constexpr int CAP = 3 * PT;                     // colidx entries staged per tile (weighted: CAP / 2, and their weights)
     static constexpr int HUB_DEG = 512;
     static constexpr int KBLK = TR * 128;                  // bytes of one K-block (32 fp32) of the A operand
     static constexpr int P_X = 0;                          // raw S_k (= hi operand) -> I_{k+1} raw (= hi operand of GEMM2)
     static constexpr int P_L = 2 * KBLK;                   // lo operand -> S' -> AI * S' -> lo of I_{k+1} -> I'_{k+1} staging
     static constexpr int P_MBAR = 4 * KBLK;                // GEMM mbarrier (8) + row-pair counter (4) + pad (4) + S-load mbarrier (8)
+                                                           // + weighted: the coming tile's weights, edge_w + inst_e0[inst] + ebase (8)
     static constexpr int P_META = P_MBAR + 32;             // DTileMeta of the coming tile (48 B)
     static constexpr int P_BG = P_META + 48;               // beta[TR], gamma[TR]
     static constexpr int P_RP = P_BG + 2 * TR * 4;         // rowptr slice [TR + 1] (+pad, hub mask)
@@ -90,35 +91,38 @@ __device__ __forceinline__ float4 tf32_unpack4(float4 p) {
 }
 
 // neighbour sum specialised by the pair's larger degree: 1..MAXR rows in one round trip, longer rows in rounds of 8
-template <int MAXR>
-__device__ __forceinline__ float4 gather_smem_zm(const float* __restrict__ lane_base, const int* cp, int deg, int zrow, uint64_t pol) {
+// (W: weighted, the weight of neighbour j at wp[j])
+template <int MAXR, bool W = false>
+__device__ __forceinline__ float4 gather_smem_zm(const float* __restrict__ lane_base, const int* cp, int deg, int zrow, uint64_t pol,
+                                                 const float* wp = nullptr) {
     const int degm = max(deg, __shfl_xor_sync(0xffffffffu, deg, 16));
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     int j = 0;
-    for (; degm - j > MAXR; j += 8) gather_exact<8>(acc, lane_base, cp, j, deg, zrow, pol);
+    for (; degm - j > MAXR; j += 8) gather_exact<8, W>(acc, lane_base, cp, j, deg, zrow, pol, wp);
     switch (degm - j) {
-        case 12: if (MAXR >= 12) gather_exact<12>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 11: if (MAXR >= 11) gather_exact<11>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 10: if (MAXR >= 10) gather_exact<10>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 9: if (MAXR >= 9) gather_exact<9>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 8: gather_exact<8>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 7: gather_exact<7>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 6: gather_exact<6>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 5: gather_exact<5>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 4: gather_exact<4>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 3: gather_exact<3>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 2: gather_exact<2>(acc, lane_base, cp, j, deg, zrow, pol); break;
-        case 1: gather_exact<1>(acc, lane_base, cp, j, deg, zrow, pol); break;
+        case 12: if (MAXR >= 12) gather_exact<12, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 11: if (MAXR >= 11) gather_exact<11, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 10: if (MAXR >= 10) gather_exact<10, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 9: if (MAXR >= 9) gather_exact<9, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 8: gather_exact<8, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 7: gather_exact<7, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 6: gather_exact<6, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 5: gather_exact<5, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 4: gather_exact<4, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 3: gather_exact<3, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 2: gather_exact<2, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
+        case 1: gather_exact<1, W>(acc, lane_base, cp, j, deg, zrow, pol, wp); break;
         default: break;
     }
     return acc;
 }
 
 // four-row item: the lane's chunks of two rows of at most D neighbours each, all 2 D loads in one round trip; each row is
-// summed alone in ascending column order (slots past its degree read the all-zero row: + 0 is exact)
-template <int D>
+// summed alone in ascending column order (slots past its degree read the all-zero row: + 0 is exact; W: weighted, the
+// weights at wpa / wpb are read after the loads are issued, pad slots weigh 0)
+template <int D, bool W = false>
 __device__ __forceinline__ void gather_two_rows(const float* __restrict__ lane_base, const int* cpa, int da, const int* cpb, int db,
-                                                int zrow, uint64_t pol, float4& sa, float4& sb) {
+                                                int zrow, uint64_t pol, float4& sa, float4& sb, const float* wpa, const float* wpb) {
     float4 v[2 * D + 1];
 #pragma unroll
     for (int k = 0; k < D; ++k) {
@@ -132,20 +136,28 @@ __device__ __forceinline__ void gather_two_rows(const float* __restrict__ lane_b
     }
     sa = make_float4(0.f, 0.f, 0.f, 0.f); sb = sa;
 #pragma unroll
-    for (int k = 0; k < D; ++k) add4(sa, v[k]);
+    for (int k = 0; k < D; ++k) {
+        if (W) v[k] = mul4(k < da ? wpa[k] : 0.f, v[k]);
+        add4(sa, v[k]);
+    }
 #pragma unroll
-    for (int k = 0; k < D; ++k) add4(sb, v[D + k]);
+    for (int k = 0; k < D; ++k) {
+        if (W) v[D + k] = mul4(k < db ? wpb[k] : 0.f, v[D + k]);
+        add4(sb, v[D + k]);
+    }
 }
+template <bool W = false>
 __device__ __forceinline__ void gather_quad(const float* __restrict__ lane_base, const int* cpa, int da, const int* cpb, int db,
-                                            int dmax, int zrow, uint64_t pol, float4& sa, float4& sb) {
+                                            int dmax, int zrow, uint64_t pol, float4& sa, float4& sb,
+                                            const float* wpa = nullptr, const float* wpb = nullptr) {
     sa = make_float4(0.f, 0.f, 0.f, 0.f); sb = sa;
     switch (dmax) {                                      // warp-uniform
-        case 6: gather_two_rows<6>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb); break;
-        case 5: gather_two_rows<5>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb); break;
-        case 4: gather_two_rows<4>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb); break;
-        case 3: gather_two_rows<3>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb); break;
-        case 2: gather_two_rows<2>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb); break;
-        case 1: gather_two_rows<1>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb); break;
+        case 6: gather_two_rows<6, W>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb, wpa, wpb); break;
+        case 5: gather_two_rows<5, W>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb, wpa, wpb); break;
+        case 4: gather_two_rows<4, W>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb, wpa, wpb); break;
+        case 3: gather_two_rows<3, W>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb, wpa, wpb); break;
+        case 2: gather_two_rows<2, W>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb, wpa, wpb); break;
+        case 1: gather_two_rows<1, W>(lane_base, cpa, da, cpb, db, zrow, pol, sa, sb, wpa, wpb); break;
         default: break;
     }
 }
@@ -169,10 +181,17 @@ struct SStep {
 // trials_table_kernel: the S_0 tile is synthesised in shared memory, the neighbour sum is the same sequence of additions
 // over the two possible I'_0 rows (bitwise the gather of the encoder's I'_0 plane), I_0 / I'_0 / hid(R_0) / probs[0] come
 // from the table. Neither y_0 nor I'_0 is ever written: the launch stores y_1, I'_1, hid(I_1), hid(R_1), beta / gamma.
+// OPT bit 8 (WGT): weighted neighbour sum AI[r] = sum over stored (r, c), ascending c, of fl(w_rc I'[c]) -- every product
+// rounded on its own (mul4), then added in the binary kernel's order, so w = 1 gives the binary bits and w = 0 those of a
+// graph without the entry. The staged window holds CAP / 2 column indices and their CAP / 2 weights; rows past it take the
+// global-list path (column indices and weights from global memory), as rows past the whole window do in the binary kernel.
 template <bool FAST, bool PERSIST, bool RF, int OPT>
 __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_constant__ StepArgs a) {
     using C = StreamCfg;
     constexpr bool ZS = (OPT & 128) != 0;
+    constexpr bool WGT = (OPT & 256) != 0;
+    static_assert(!(ZS && WGT), "step 0 from descriptors is not weighted");
+    constexpr int CAPS = WGT ? C::CAP / 2 : C::CAP;                   // column indices staged per tile
     static_assert(!ZS || (RF && !PERSIST && (OPT & 64)), "step 0 from descriptors: inference without an R plane, one launch, raw S tile");
     constexpr int PT = C::PT, TR = C::TR, RSTEP = C::RSTEP, PASS = C::PASS;
     // The dynamic shared memory of this kernel starts at a 1024-byte boundary of the shared window (declared so, and
@@ -202,6 +221,8 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
     float* hs_s = reinterpret_cast<float*>(hb + C::P_HS);
     float* hr_s = reinterpret_cast<float*>(hb + C::P_HR);
     int* ci_s = reinterpret_cast<int*>(hb + C::P_CI);
+    const float* wt_s = reinterpret_cast<const float*>(ci_s + CAPS);  // WGT: the staged entries' weights
+    const float** wslot = reinterpret_cast<const float**>(hb + C::P_MBAR + 24);   // WGT: weights of the tile's entries
     unsigned* hub_mask = reinterpret_cast<unsigned*>(rp_s + TR + 2);
     const uint32_t* items_s = reinterpret_cast<const uint32_t*>(hb + C::P_PM);
     unsigned char* kind_s = hb + C::P_ZK;                             // ZS: 1 = seed row
@@ -242,6 +263,7 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
             m.colidx = I.colidx;
         }
         *meta = m;
+        if (WGT && seq < n_tiles) *wslot = a.edge_w + a.inst_e0[m.inst0] + m.ebase;
     };
     // the same thread: request the S_k rows of that tile (raw fp32, operand layout) into Xs
     auto issue_s_load = [&]() {
@@ -351,11 +373,17 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
             float bgv = 0.f;
             uint32_t pmv = 0;
             if (!ZS && single && t < 64) pmv = __ldg(reinterpret_cast<const uint32_t*>(a.bv.tile_perm) + (size_t)(tile0 / TR) * 64 + t);
-            const int ecnt = min(m.ecnt, C::CAP);
+            const int ecnt = min(m.ecnt, CAPS);
+            // slot i of the window: column index i (i < CAPS) or, weighted, the weight of entry i - CAPS
+            auto staged = [&](int i) { return i < CAPS ? i < ecnt : (WGT && i - CAPS < ecnt); };
             if (single && t <= nrows) rpv = __ldg(m.rowptr + t);
             if (single) {
 #pragma unroll
-                for (int u = 0; u < 3; ++u) if (t + u * PT < ecnt) civ[u] = __ldg(m.colidx + ebase + t + u * PT);
+                for (int u = 0; u < 3; ++u) {
+                    const int i = t + u * PT;
+                    if (i < CAPS) { if (i < ecnt) civ[u] = __ldg(m.colidx + ebase + i); }
+                    else if (staged(i)) civ[u] = __float_as_int(__ldg(*wslot + (i - CAPS)));
+                }
             }
             if (!ZS && t >= PT / 2 && t < PT / 2 + nrows) bgv = a.beta[tile0 + t - PT / 2];
             if (!ZS && t >= 3 * PT / 4 && t < 3 * PT / 4 + nrows) bgv = a.gamma[tile0 + t - 3 * PT / 4];
@@ -395,7 +423,7 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
             if (!ZS && single && t < 64) reinterpret_cast<uint32_t*>(hb + C::P_PM)[t] = pmv;
             if (single) {
 #pragma unroll
-                for (int u = 0; u < 3; ++u) if (t + u * PT < ecnt) ci_s[t + u * PT] = civ[u];   // instance-local ids
+                for (int u = 0; u < 3; ++u) if (staged(t + u * PT)) ci_s[t + u * PT] = civ[u];   // instance-local ids
             }
             if (!ZS && t >= PT / 2 && t < PT / 2 + nrows) bg_s[t - PT / 2] = bgv;
             if (!ZS && t >= 3 * PT / 4 && t < 3 * PT / 4 + nrows) bg_s[TR + t - 3 * PT / 4] = bgv;
@@ -433,10 +461,10 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
             const bool hubrow = relay && deg > C::HUB_DEG;                 // summed by the in-order relay below
             if (hubrow) deg = 0;
             ok = rr < nrows && !hubrow;
-            const int over = (e_rel + deg > C::CAP) ? 1 : 0;
+            const int over = (e_rel + deg > CAPS) ? 1 : 0;
             if (__any_sync(0xffffffffu, over))               // indices beyond the staged slice: same gather on the global list
-                return gather_smem_zm<12>(lane_base, m.colidx + ebase + e_rel, deg, zrow, pol_keep);
-            return gather_smem_zm<12>(lane_base, ci_s + e_rel, deg, zrow, pol_keep);
+                return gather_smem_zm<12, WGT>(lane_base, m.colidx + ebase + e_rel, deg, zrow, pol_keep, WGT ? *wslot + e_rel : nullptr);
+            return gather_smem_zm<12, WGT>(lane_base, ci_s + e_rel, deg, zrow, pol_keep, WGT ? wt_s + e_rel : nullptr);
         };
         umma::mbar_wait_suspend(mbar, phase); phase ^= 1;
         umma::fence_after_sync();
@@ -609,7 +637,13 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
                         int dmax = max(da, db);
                         dmax = max(dmax, __shfl_xor_sync(0xffffffffu, dmax, 16));
                         float4 sa, sb;
-                        gather_quad(lane_base, ci_s + ea, da, ci_s + eb, db, dmax, zrow, pol_keep, sa, sb);
+                        if (!WGT) gather_quad(lane_base, ci_s + ea, da, ci_s + eb, db, dmax, zrow, pol_keep, sa, sb);
+                        else if (__any_sync(0xffffffffu, ea + da > CAPS || eb + db > CAPS)) {   // past the halved window
+                            const float* wt = *wslot;
+                            gather_quad<true>(lane_base, m.colidx + ebase + ea, da, m.colidx + ebase + eb, db, dmax, zrow, pol_keep,
+                                              sa, sb, wt + ea, wt + eb);
+                        } else
+                            gather_quad<true>(lane_base, ci_s + ea, da, ci_s + eb, db, dmax, zrow, pol_keep, sa, sb, wt_s + ea, wt_s + eb);
                         finish_row(ra, oka, sa);
                         finish_row(rb, okb, sb);
                     } else {
@@ -637,6 +671,7 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
                             mm &= mm - 1;
                             const int dg = rp_s[r + 1] - rp_s[r];
                             const int* cp = m.colidx + rp_s[r];
+                            const float* wp = WGT ? *wslot + (rp_s[r] - ebase) : nullptr;
                             const int n_sr = (dg + SR - 1) / SR;
 #pragma unroll 1
                             for (int sr = 0; sr < n_sr; ++sr) {
@@ -646,6 +681,10 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
                                 for (int k = 0; k < 8; ++k) {
                                     const int c = (j0 + k < dg) ? cp[j0 + k] : zrow;
                                     v[k] = ldg4_hint(lane_base + (size_t)(unsigned)c * H, pol_keep);
+                                }
+                                if (WGT) {                                   // products before the relayed adds
+#pragma unroll
+                                    for (int k = 0; k < 8; ++k) v[k] = mul4((j0 + k < dg) ? wp[j0 + k] : 0.f, v[k]);
                                 }
                                 if (warp > 0) umma::mbar_wait(&hbar[warp], (uint32_t)(nsr_done & 1));
                                 else if (nsr_done > 0) umma::mbar_wait(&hbar[0], (uint32_t)((nsr_done - 1) & 1));
@@ -692,7 +731,8 @@ __global__ void __launch_bounds__(D_THREADS, 1) step_stream_kernel(const __grid_
                         e0 = I.rowptr[g - row0];
                         deg = I.rowptr[g - row0 + 1] - e0;
                     }
-                    const float4 acc = gather_row(STP(ip_in), ci, e0, deg, row0, l, lane);
+                    const float4 acc = gather_row<WGT>(STP(ip_in), ci, e0, deg, row0, l, lane,
+                                                       WGT ? a.edge_w + a.inst_e0[inst] : nullptr);
                     finish_row(rr, rr < nrows, acc);
                 }
             }

@@ -105,12 +105,15 @@ __device__ __forceinline__ int find_instance(const GnBatchView& bv, int64_t r) {
 // Sequential ascending-column neighbour sum of one row by a half-warp (lane l owns 16 B of
 // the row); both half-warps of the warp iterate together (trip count = max of the two
 // degrees) so that full-mask shuffles stay convergent. 8 neighbour rows in flight per lane.
+// W: weighted sum, acc += fl(w_e src[c_e]) with w_e = wp[e0 + j] (the entries' weights in CSR order).
+template <bool W = false>
 __device__ __forceinline__ float4 gather_row(const float* __restrict__ src, const int32_t* ci, int e0, int deg,
-                                              int row0, int l, int lane) {
+                                              int row0, int l, int lane, const float* wp = nullptr) {
     const int degmax = max(deg, __shfl_xor_sync(0xffffffffu, deg, 16));
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int eb = 0; eb < degmax; eb += 16) {
         const int mine = (eb + l < deg) ? ci[e0 + eb + l] + row0 : -1;
+        const float mw = (W && eb + l < deg) ? wp[e0 + eb + l] : 0.f;
 #pragma unroll
         for (int jb = 0; jb < 16; jb += 8) {
             if (eb + jb < degmax) {
@@ -119,6 +122,10 @@ __device__ __forceinline__ float4 gather_row(const float* __restrict__ src, cons
                 for (int j = 0; j < 8; ++j) {
                     const int c = __shfl_sync(0xffffffffu, mine, (lane & 16) + jb + j);
                     v[j] = (c >= 0) ? ldg4(src + (size_t)c * H + 4 * l) : make_float4(0.f, 0.f, 0.f, 0.f);
+                }
+                if (W) {
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) v[j] = mul4(__shfl_sync(0xffffffffu, mw, (lane & 16) + jb + j), v[j]);
                 }
 #pragma unroll
                 for (int j = 0; j < 8; ++j) add4(acc, v[j]);

@@ -26,8 +26,10 @@ class DeviceGraph:
         indptr = np.ascontiguousarray(A.indptr, dtype=np.int32)
         indices = np.asarray(A.indices[:indptr[-1]], dtype=np.int32)
         rows = np.repeat(np.arange(self.n, dtype=np.int32), np.diff(indptr))
-        indices = np.ascontiguousarray(indices[np.lexsort((indices, rows))])      # per-row column sort
+        order = np.lexsort((indices, rows))                                      # per-row column sort
+        indices = np.ascontiguousarray(indices[order])
         self.indptr, self.indices = indptr, indices
+        self._values = np.asarray(A.data[:indptr[-1]])[order]
         self.nnz = int(indptr[-1])
         h = ctypes.c_void_p()
         L = _lib.lib()
@@ -43,6 +45,10 @@ class DeviceGraph:
     def edges(self):
         """(row, col) of every stored entry, int64, in the order of the edge gradients (rollout's edge_weight)."""
         return np.repeat(np.arange(self.n, dtype=np.int64), np.diff(self.indptr)), self.indices.astype(np.int64)
+
+    def edge_values(self):
+        """A's stored values (float32) in edges() order: a weighted matrix's weights as rollout's contact_weight."""
+        return self._values.astype(np.float32)
 
     def __del__(self):
         try:

@@ -103,27 +103,31 @@ class ODEBlock(nn.Module):
             probs = probs + 0.0 * (self.odefunc.ln.weight.sum() + self.odefunc.ln.bias.sum())
         return probs
 
-    def rollout_probs(self, x, out_steps=None, instances=None, *, edge_weight=None):
+    def rollout_probs(self, x, out_steps=None, instances=None, *, edge_weight=None, contact_weight=None):
         """x [sum N, 3+H] -> probabilities [T (or len(out_steps)), sum N, 3]. `instances` (graph index per instance)
         spares the marker column's device read when the caller knows its batch. edge_weight: all-ones CUDA tensor of the
         batch's nnz (instance after instance, each in its graph's DeviceGraph.edges() order); when it requires grad it
-        receives dL/dw of every stored adjacency entry."""
+        receives dL/dw of every stored adjacency entry. contact_weight: the weights the neighbour sum runs with, same
+        layout, any finite values; when it requires grad it receives dL/dw at those weights."""
         batch = self.odefunc.batch_from_instances(instances) if instances is not None \
             else self.odefunc.batch_from_markers(x[:, 5])
         if batch.M != x.size(0):
             raise RuntimeError("batch of %d rows for an input of %d rows" % (batch.M, x.size(0)))
-        return self._finish(_ro.rollout(x, batch, self._dt, self._params(), self.grad_mode, out_steps, edge_weight))
+        return self._finish(_ro.rollout(x, batch, self._dt, self._params(), self.grad_mode, out_steps, edge_weight,
+                                        contact_weight))
 
-    def forward(self, x, instances=None, *, edge_weight=None):
-        S, I, R = self.rollout_probs(x, instances=instances, edge_weight=edge_weight).chunk(3, dim=-1)
+    def forward(self, x, instances=None, *, edge_weight=None, contact_weight=None):
+        S, I, R = self.rollout_probs(x, instances=instances, edge_weight=edge_weight,
+                                    contact_weight=contact_weight).chunk(3, dim=-1)
         return S, I, R
 
-    def forward_trials(self, instances, seeds, beta, gamma, out_steps=None, *, edge_weight=None):
+    def forward_trials(self, instances, seeds, beta, gamma, out_steps=None, *, edge_weight=None, contact_weight=None):
         """Rollout from compact descriptors (N4): instance i runs on graph instances[i] with seeds[i], beta[i], gamma[i]
         (replaces the dense per-instance blocks of ode_nn_ngraphs.py:326-345). Returns (S, I, R). beta / gamma given as
-        tensors that require grad receive dL/dbeta[i], dL/dgamma[i]; edge_weight as in rollout_probs."""
+        tensors that require grad receive dL/dbeta[i], dL/dgamma[i]; edge_weight and contact_weight as in rollout_probs."""
         batch = self.odefunc.batch_from_instances(instances)
         trials = _ro.TrialSet(seeds, beta, gamma, batch.sizes, self.linearS1.weight.device)
         probs = self._finish(_ro.rollout_trials(batch, trials, self._dt, self._params(), self.grad_mode, out_steps,
-                                                beta=beta, gamma=gamma, edge_weight=edge_weight))
+                                                beta=beta, gamma=gamma, edge_weight=edge_weight,
+                                                contact_weight=contact_weight))
         return probs.chunk(3, dim=-1)

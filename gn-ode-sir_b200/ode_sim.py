@@ -95,29 +95,34 @@ class ODEBlock(nn.Module):
             probs = probs + 0.0 * (self.odefunc.ln.weight.sum() + self.odefunc.ln.bias.sum())
         return probs
 
-    def rollout_probs(self, x, out_steps=None, *, edge_weight=None):
+    def rollout_probs(self, x, out_steps=None, *, edge_weight=None, contact_weight=None):
         """x [B, N, 3+H] -> probabilities [T (or len(out_steps)), B*N, 3] in one tensor. edge_weight: all-ones [B, nnz]
         CUDA tensor (trial b's edges in odefunc.device_graph().edges() order); when it requires grad it receives dL/dw of
-        every edge of every trial."""
+        every edge of every trial. contact_weight: [B, nnz] weights the neighbour sum runs with (one weight vector per trial,
+        any finite values; DeviceGraph.edge_values() for a weighted matrix); when it requires grad it receives dL/dw."""
         x = x.view(-1, x.size(-1))                     # [B*N, 3+H]
         n_trials = x.size(0) // self.odefunc.device_graph().n
         batch = self.odefunc.batch_for(n_trials)
-        return self._finish(_ro.rollout(x, batch, self._dt, self._params(), self.grad_mode, out_steps, edge_weight))
+        return self._finish(_ro.rollout(x, batch, self._dt, self._params(), self.grad_mode, out_steps, edge_weight,
+                                        contact_weight))
 
-    def forward(self, x, *, edge_weight=None):
-        S, I, R = self.rollout_probs(x, edge_weight=edge_weight).chunk(3, dim=-1)          # each [T, M, 1]
+    def forward(self, x, *, edge_weight=None, contact_weight=None):
+        S, I, R = self.rollout_probs(x, edge_weight=edge_weight,
+                                    contact_weight=contact_weight).chunk(3, dim=-1)          # each [T, M, 1]
         return S, I, R
 
-    def forward_trials(self, seeds, beta, gamma, out_steps=None, probs_out=None, workspace=None, *, edge_weight=None):
+    def forward_trials(self, seeds, beta, gamma, out_steps=None, probs_out=None, workspace=None, *, edge_weight=None,
+                       contact_weight=None):
         """The same rollout from compact trial descriptors (N4): seeds[i] = node ids infected at t = 0 in trial i,
         beta[i], gamma[i] -- instead of the dense [N, 3+H] block per trial main() builds (ode_nn_ngraph_sim.py:371-390).
         Returns (S, I, R), each [T (or len(out_steps)), B*N, 1]. beta / gamma given as tensors that require grad receive
-        dL/dbeta[i], dL/dgamma[i] (calibration of a trial through the trained model); edge_weight as in rollout_probs."""
+        dL/dbeta[i], dL/dgamma[i] (calibration of a trial through the trained model); edge_weight and contact_weight as in
+        rollout_probs."""
         is_set = isinstance(seeds, _ro.TrialSet)                      # a prepared (device-resident) descriptor set
         batch = self.odefunc.batch_for(seeds.n_inst if is_set else len(seeds))
         dev = self.linearS1.weight.device
         trials = seeds if is_set else _ro.TrialSet(seeds, beta, gamma, batch.sizes, dev)
         probs = self._finish(_ro.rollout_trials(batch, trials, self._dt, self._params(), self.grad_mode, out_steps,
                                                 probs_out, workspace, *((None, None) if is_set else (beta, gamma)),
-                                                edge_weight=edge_weight))
+                                                edge_weight=edge_weight, contact_weight=contact_weight))
         return probs.chunk(3, dim=-1)

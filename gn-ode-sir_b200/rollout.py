@@ -94,7 +94,9 @@ def dt_array(integration_time):
 
 class _Rollout(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, batch, dt, grad_mode, want_grad, out_steps, edge_weight, *params):
+    def forward(ctx, x, batch, dt, grad_mode, want_grad, out_steps, weighted, edge_weight, *params):
+        # edge_weight: None, the unit weights of rollout(edge_weight=) (binary forward) or, weighted, the contact weights
+        # of rollout(contact_weight=) that the neighbour sum multiplies; when it requires grad it receives dL/dw
         L = _lib.lib()
         M, T = batch.M, len(dt) + 1
         steps, steps_p, n_out = _steps_arg(out_steps, T)
@@ -106,7 +108,8 @@ class _Rollout(torch.autograd.Function):
             _check_cuda_f32(p, k)
             ps.append(p.detach().contiguous())
         # grad mode is always off inside forward(): the caller's grad mode arrives as `want_grad`
-        need_grad = bool(want_grad) and (ctx.needs_input_grad[0] or any(ctx.needs_input_grad[6:]))
+        need_grad = bool(want_grad) and (ctx.needs_input_grad[0] or any(ctx.needs_input_grad[7:]))
+        ew = edge_weight.detach().contiguous() if weighted else None
         with torch.cuda.device(x.device):
             traj = torch.empty((T, 3, M, H), dtype=torch.float32, device=x.device) if need_grad else None
             probs = torch.empty((n_out, M, 3), dtype=torch.float32, device=x.device)
@@ -121,24 +124,27 @@ class _Rollout(torch.autograd.Function):
                     aux = torch.empty(int(L.gnode_rollout_aux_bytes(batch.handle, T)) // 4, dtype=torch.float32, device=x.device)
                 except torch.cuda.OutOfMemoryError:          # 2/3 of the trajectory's size on top of it: optional
                     aux = None
-            _lib.check(L.gnode_rollout_forward_aux(batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T,
-                                                   dt.ctypes.data_as(_lib.c_float_p), steps_p, n_out,
-                                                   _ptr(traj) if need_grad else None,
-                                                   _ptr(aux) if aux is not None else None, ctypes.byref(filled),
-                                                   _ptr(probs), _ptr(ws), ws_bytes,
-                                                   _stream(x.device)), "gnode_rollout_forward_aux")
+            args = (batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T, dt.ctypes.data_as(_lib.c_float_p),
+                    steps_p, n_out, _ptr(traj) if need_grad else None, _ptr(aux) if aux is not None else None,
+                    ctypes.byref(filled), _ptr(probs))
+            if weighted:
+                _lib.check(L.gnode_rollout_forward_weighted(*args, _ptr(ew), _ptr(ws), ws_bytes, _stream(x.device)),
+                           "gnode_rollout_forward_weighted")
+            else:
+                _lib.check(L.gnode_rollout_forward_aux(*args, _ptr(ws), ws_bytes, _stream(x.device)),
+                           "gnode_rollout_forward_aux")
         if need_grad:
-            ctx.save_for_backward(x, traj, *ps)
+            ctx.save_for_backward(x, traj, ew, *ps)
             ctx.batch, ctx.dt, ctx.grad_mode, ctx.steps = batch, dt, grad_mode, steps
             ctx.edge_shape = tuple(edge_weight.shape) if edge_weight is not None else None
             ctx.aux = aux if filled.value == 1 else None
-            ctx.wgrad = any(ctx.needs_input_grad[7:])       # False: input gradients only (no weight-gradient phase)
+            ctx.wgrad = any(ctx.needs_input_grad[8:])       # False: input gradients only (no weight-gradient phase)
         return probs
 
     @staticmethod
     def backward(ctx, grad_probs):
         L = _lib.lib()
-        x, traj, *ps = ctx.saved_tensors
+        x, traj, ew, *ps = ctx.saved_tensors
         batch, dt = ctx.batch, ctx.dt
         T = len(dt) + 1
         grad_probs = grad_probs.contiguous()
@@ -150,28 +156,30 @@ class _Rollout(torch.autograd.Function):
             # dL/dx: columns 0..4 written by the sweep, the others (graph marker, unused bg channels) carry no gradient
             grad_x = torch.zeros(tuple(x.shape), dtype=torch.float32, device=x.device) if ctx.needs_input_grad[0] else None
             # dL/dw per stored adjacency entry (one float more than nnz keeps the pointer valid on edgeless batches)
-            grad_edge = torch.empty(batch.nnz + 1, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[6] else None
-            ws_bytes = int(L.gnode_backward_workspace_bytes(batch.handle))
+            grad_edge = torch.empty(batch.nnz + 1, dtype=torch.float32, device=x.device) if ctx.needs_input_grad[7] else None
+            ws_bytes = int(L.gnode_backward_weighted_workspace_bytes(batch.handle) if ew is not None
+                           else L.gnode_backward_workspace_bytes(batch.handle))
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
             pstruct = _params_struct(ps)
             mode = {"adjoint": _lib.GRAD_ADJOINT, "discrete": _lib.GRAD_DISCRETE}[ctx.grad_mode]
-            _lib.check(L.gnode_rollout_backward_edges(batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T,
-                                                      dt.ctypes.data_as(_lib.c_float_p), _ptr(traj),
-                                                      _ptr(ctx.aux) if ctx.aux is not None else None, _ptr(grad_probs),
-                                                      steps_p, len(steps) if steps is not None else 0, mode,
-                                                      _ptr(grads) if grads is not None else None,
-                                                      _ptr(grad_x) if grad_x is not None else None,
-                                                      grad_x.stride(0) if grad_x is not None else 0,
-                                                      _ptr(grad_edge) if grad_edge is not None else None,
-                                                      _ptr(ws), ws_bytes, _stream(x.device)),
-                       "gnode_rollout_backward_edges")
+            args = (batch.handle, _ptr(x), x.stride(0), ctypes.byref(pstruct), T, dt.ctypes.data_as(_lib.c_float_p),
+                    _ptr(traj), _ptr(ctx.aux) if ctx.aux is not None else None, _ptr(grad_probs), steps_p,
+                    len(steps) if steps is not None else 0, mode, _ptr(grads) if grads is not None else None,
+                    _ptr(grad_x) if grad_x is not None else None, grad_x.stride(0) if grad_x is not None else 0,
+                    _ptr(grad_edge) if grad_edge is not None else None)
+            if ew is not None:
+                _lib.check(L.gnode_rollout_backward_weighted(*args, _ptr(ew), _ptr(ws), ws_bytes, _stream(x.device)),
+                           "gnode_rollout_backward_weighted")
+            else:
+                _lib.check(L.gnode_rollout_backward_edges(*args, _ptr(ws), ws_bytes, _stream(x.device)),
+                           "gnode_rollout_backward_edges")
         out, off = [], 0
         for i, (k, shape) in enumerate(_lib.GRAD_LAYOUT):
             n = int(np.prod(shape))
-            out.append(grads[off:off + n].view(shape) if ctx.needs_input_grad[7 + i] else None)
+            out.append(grads[off:off + n].view(shape) if ctx.needs_input_grad[8 + i] else None)
             off += n
         ge = grad_edge[:batch.nnz].view(ctx.edge_shape) if grad_edge is not None else None
-        return (grad_x, None, None, None, None, None, ge, *out)
+        return (grad_x, None, None, None, None, None, None, ge, *out)
 
 
 def _check_edge_weight(edge_weight, batch):
@@ -186,19 +194,40 @@ def _check_edge_weight(edge_weight, batch):
                          "receives dL/dw; to remove an edge, build a graph without it")
 
 
-def rollout(x, batch, dt, params, grad_mode="adjoint", out_steps=None, edge_weight=None):
+def _check_contact_weight(contact_weight, batch, edge_weight):
+    """contact_weight: the weight of every stored adjacency entry of the batch, any finite float32 values on the
+    batch's device (one device-wide finiteness check per call)."""
+    if edge_weight is not None:
+        raise ValueError("pass either edge_weight (unit weights that receive dL/dw of the binary rollout) or "
+                         "contact_weight (the weights the rollout runs with, which receive dL/dw themselves), not both")
+    _check_cuda_f32(contact_weight, "contact_weight")
+    if contact_weight.numel() != batch.nnz:
+        raise ValueError("contact_weight must hold one value per stored adjacency entry of the batch (%d), got %d"
+                         % (batch.nnz, contact_weight.numel()))
+    if not bool(torch.isfinite(contact_weight.detach()).all()):
+        raise ValueError("contact_weight must be finite")
+
+
+def rollout(x, batch, dt, params, grad_mode="adjoint", out_steps=None, edge_weight=None, contact_weight=None):
     """x [M, >=5] -> probabilities [T, M, 3] (or [len(out_steps), M, 3]: only those grid points are decoded and
     stored); params in PARAM_ORDER (state_dict names). Differentiable with respect to the parameters and to x (columns
     S0, I0, R0, beta, gamma; the other columns get zero gradients). edge_weight: an all-ones float32 CUDA tensor with
     batch.nnz elements (instance after instance, each in DeviceGraph.edges() order); when it requires grad it receives
-    dL/dw of every stored adjacency entry, the gradient of the weighted neighbour sum at w = 1."""
+    dL/dw of every stored adjacency entry, the gradient of the weighted neighbour sum at w = 1.
+    contact_weight: a float32 CUDA tensor with batch.nnz elements in the same order (DeviceGraph.edge_values() gives a
+    weighted matrix's stored values in that order), any finite values: the neighbour sum becomes
+    AI[r] = sum over stored (r, c) of w_rc I'[c] (ones give the binary rollout's bits, a zero the bits of a graph without
+    that entry). When it requires grad it receives dL/dw at those weights. Not together with edge_weight."""
     if grad_mode not in ("adjoint", "discrete"):
         raise ValueError("grad_mode must be 'adjoint' or 'discrete'")
-    if edge_weight is not None:
+    if contact_weight is not None:
+        _check_contact_weight(contact_weight, batch, edge_weight)
+        edge_weight = contact_weight
+    elif edge_weight is not None:
         _check_edge_weight(edge_weight, batch)
     want_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params) or
                                              (edge_weight is not None and edge_weight.requires_grad))
-    return _Rollout.apply(x, batch, dt, grad_mode, want_grad, out_steps, edge_weight, *params)
+    return _Rollout.apply(x, batch, dt, grad_mode, want_grad, out_steps, contact_weight is not None, edge_weight, *params)
 
 
 class TrialSet:
@@ -292,18 +321,23 @@ class _ExpandTrials(torch.autograd.Function):
 
 
 def rollout_trials(batch, trials, dt, params, grad_mode="adjoint", out_steps=None, probs_out=None, workspace=None,
-                   beta=None, gamma=None, edge_weight=None):
+                   beta=None, gamma=None, edge_weight=None, contact_weight=None):
     """Rollout straight from compact trial descriptors. Without gradients: ONE C-ABI call (expansion into the
     workspace + rollout), optionally into caller-owned `probs_out` / `workspace` buffers (streaming loops reuse them).
     With gradients: the compact x is kept for the reverse sweep. `beta` / `gamma`: the tensors the set was made from;
     when one of them requires grad, it receives dL/dbeta[i] (dL/dgamma[i]) per instance. Seed sets are discrete and
-    have no gradient. `edge_weight`: as for rollout() ([B, nnz] for B trials of one graph)."""
-    if edge_weight is not None:
+    have no gradient. `edge_weight`, `contact_weight`: as for rollout() ([B, nnz] for B trials of one graph). With
+    contact weights the descriptors are expanded into x and the rollout runs from it (the fused descriptor-fed Euler
+    step 0 is binary)."""
+    if contact_weight is not None:
+        _check_contact_weight(contact_weight, batch, edge_weight)
+    elif edge_weight is not None:
         _check_edge_weight(edge_weight, batch)
     want_x = torch.is_grad_enabled() and any(torch.is_tensor(v) and v.requires_grad for v in (beta, gamma))
+    ew = contact_weight if contact_weight is not None else edge_weight
     want_grad = want_x or (torch.is_grad_enabled() and (any(p.requires_grad for p in params) or
-                                                        (edge_weight is not None and edge_weight.requires_grad)))
-    if want_grad:
+                                                        (ew is not None and ew.requires_grad)))
+    if want_grad or contact_weight is not None:
         if want_x:
             bt = beta if torch.is_tensor(beta) else trials.beta
             gt = gamma if torch.is_tensor(gamma) else trials.gamma
@@ -312,7 +346,11 @@ def rollout_trials(batch, trials, dt, params, grad_mode="adjoint", out_steps=Non
             x = _ExpandTrials.apply(bt, gt, batch, trials)
         else:
             x = expand_trials(batch, trials)
-        return rollout(x, batch, dt, params, grad_mode, out_steps, edge_weight)
+        probs = rollout(x, batch, dt, params, grad_mode, out_steps, edge_weight, contact_weight)
+        if probs_out is not None and not want_grad:
+            probs_out.copy_(probs)
+            return probs_out
+        return probs
     L = _lib.lib()
     if trials.n_inst != len(batch.sizes):
         raise ValueError("%d trial descriptors for a batch of %d instances" % (trials.n_inst, len(batch.sizes)))

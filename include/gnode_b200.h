@@ -121,7 +121,8 @@ int64_t gnode_launch_count(void);
  * ODEfunc.A_list (ode_nn_ngraph_sim.py:41, ode_nn_ngraphs.py:41, built by
  * nx.adjacency_matrix at ode_nn.py:413) and its per-step re-expansion to COO.
  * rowptr[n+1], colidx[nnz] are HOST int32 CSR arrays; stored values are ignored
- * (every stored entry counts once, as in the reference). Columns are sorted per
+ * (every stored entry counts once, as in the reference; per-edge weights are passed to
+ * the _weighted rollout calls instead, see below). Columns are sorted per
  * row at creation so the neighbour sum runs in ascending-column order, the order
  * of the reference's CPU scatter_add_. The transposed pattern is built here too
  * (backward); undirected graphs share one copy. */
@@ -272,6 +273,33 @@ int gnode_rollout_backward_edges(gnode_batch_t b, const float* x, int64_t ldx, c
                                  const int32_t* out_steps, int32_t n_out, int32_t grad_mode, float* grads_out,
                                  float* grad_x, int64_t ldgx, float* grad_edge, void* workspace, size_t workspace_bytes,
                                  void* stream);
+
+/* ---- weighted contact graphs: per-edge weights in the neighbour sum --------------------
+ * The rollout with AI[r] = sum over stored (r, c), in ascending column order, of fl(w_rc * I'[c]): every product rounded
+ * on its own, then added in the binary sum's order. So w = 1 gives the binary rollout's bits and w = 0 those of a graph
+ * built without that entry (I' is finite). Weights may take any finite value.
+ *   edge_w  DEVICE fp32 [nnz_total], in the batch's edge order (that of grad_edge above); read at every call, so values
+ *           written in place between calls are honoured (also by a replayed reverse sweep).
+ * gnode_rollout_forward_weighted: the arguments of gnode_rollout_forward_aux plus edge_w; edge_w == NULL is that call,
+ * bit for bit. The weighted neighbour sum runs on the default step kernel (5) with tensor maps, one launch per step or
+ * the persistent cooperative launch; any other step-kernel setting, or a driver without tensor maps, returns
+ * GNODE_ERR_UNSUPPORTED. With aux, the stored AI_k is the weighted sum.
+ * gnode_rollout_backward_weighted: the arguments of gnode_rollout_backward_edges plus edge_w (the weights of the forward
+ * that stored traj / aux); grad_edge then receives dL/dw at those weights. The transposed gather of the sweep,
+ * sum_c w_cr gAI[c], reads the weights in transpose order: a kernel of the enqueued sequence permutes edge_w into the
+ * workspace by each graph's transpose map (kept at gnode_graph_create, uploaded on the first weighted call -- a blocking
+ * copy, made before any stream capture). Workspace: gnode_backward_weighted_workspace_bytes(b) (the unweighted size
+ * plus nnz_total floats). edge_w == NULL is gnode_rollout_backward_edges, bit for bit. */
+int gnode_rollout_forward_weighted(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p,
+                                   int32_t T, const float* dt_host, const int32_t* out_steps, int32_t n_out,
+                                   float* traj, float* aux, int32_t* aux_filled, float* probs, const float* edge_w,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+size_t gnode_backward_weighted_workspace_bytes(gnode_batch_t b);
+int gnode_rollout_backward_weighted(gnode_batch_t b, const float* x, int64_t ldx, const gnode_params_t* p, int32_t T,
+                                    const float* dt_host, const float* traj, const float* aux, const float* grad_probs,
+                                    const int32_t* out_steps, int32_t n_out, int32_t grad_mode, float* grads_out,
+                                    float* grad_x, int64_t ldgx, float* grad_edge, const float* edge_w, void* workspace,
+                                    size_t workspace_bytes, void* stream);
 
 /* Per-instance sums of grad_x columns 3 and 4 (instance i = rows [row0_i, row0_i + n_i)), in a fixed order:
  * the gradient of compact trial descriptors' beta[i], gamma[i] (N4). grad_beta, grad_gamma: DEVICE float[n_inst]. */
